@@ -272,6 +272,26 @@ class DeviceBatch:
                               self.n, block_size=self.block_size, stream=self.stream)
 
 
+DUMP_SEED, DUMP_SAMPLE = 20240611, 12        # 12 whole blocks as float32: 48 MiB of the at most 64 MB dumped
+
+
+def dump_outputs(path: str, d_dst, d_osz, d_st) -> None:
+    """What one batched decompression returned, as float .npy files under path, so that two builds can be
+    compared output for output: the status and output size of every block, and the bytes of the first block,
+    the last (partial) block and a fixed, seeded sample of the others."""
+    import torch
+    os.makedirs(path, exist_ok=True)
+    nblk = d_dst.shape[0]
+    rng = np.random.default_rng(DUMP_SEED)
+    inner = rng.choice(np.arange(1, nblk - 1), size=min(DUMP_SAMPLE - 2, max(nblk - 2, 0)), replace=False)
+    pick = np.unique(np.concatenate([[0, nblk - 1], inner]).astype(np.int64))
+    blocks = d_dst[torch.from_numpy(pick).to(d_dst.device)].cpu().numpy()
+    np.save(os.path.join(path, "status.npy"), d_st.cpu().numpy().astype(np.float64))
+    np.save(os.path.join(path, "out_size.npy"), d_osz.cpu().numpy().astype(np.float64))
+    np.save(os.path.join(path, "sample_index.npy"), pick.astype(np.float64))
+    np.save(os.path.join(path, "sample_blocks.npy"), blocks.astype(np.float32))
+
+
 def time_device(fn, dev, warmup: int, reps: int) -> float:
     """ms per call, CUDA events on the current (launching) stream."""
     import torch
@@ -698,7 +718,12 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-secondary", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="headline only: write what the last timed step returned (every block's status and size, a "
+                         "fixed sample of decoded blocks) to DIR/<name>.npy, from rank 0")
     args = ap.parse_args()
+    if args.dump_outputs and (args.config != 2 or args.impl != "cryogpu"):
+        ap.error("--dump-outputs applies to the headline (--config 2, --impl cryogpu)")
     args.warmup = max(args.warmup, 3) if args.impl == "cryogpu" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -779,6 +804,8 @@ def main():
         step()
         ev[k + 1].record()
     barrier()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, d_dst, d_osz, d_st)
     clocks = keep_sampling(sampler, dev, step)
     total_ms = ev[0].elapsed_time(ev[-1])
     step_ms = [ev[k].elapsed_time(ev[k + 1]) for k in range(args.steps)]
@@ -875,13 +902,14 @@ def main():
     # ---- CPU baseline beside it: the reference's compression.c on this box's cores ----
     cpu = None
     if rank == 0 and world == 1 and not args.no_cpu:
+        from oracle import ref
         threads = os.cpu_count() or 1
         sample = chunks[: min(len(chunks), max(64, threads * 16))]
         gbs_all, reps = cpu_reference_decompress(METHOD, sample, threads, 10.0)
         gbs_one, _ = cpu_reference_decompress(METHOD, sample, 1, 4.0)
         cpu = {"value": gbs_all, "unit": "GB/s", "cores": threads, "kind": "reference",
-               "sample": f"{len(sample)} of the {nblk} blocks x {reps} passes through oracle/_ref "
-                         f"(reference compression.c + libzstd 1.5.5), {threads} threads",
+               "sample": f"{len(sample)} of the {nblk} blocks x {reps} passes through {ref.describe()}, "
+                         f"{threads} threads",
                "value_1_thread": gbs_one}
 
     # ---- the rest of the metric: lz4 and zstd-1, both directions, every block kind ----

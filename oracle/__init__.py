@@ -3,8 +3,9 @@
 CPU checkers for the block-codec path of pg_cryogen:
 
 * ``oracle.ref``  -- ctypes binding of ``oracle/_ref/libcryoref.so``: the reference's
-  UNMODIFIED compression.c + storage.c (compiled from /root/reference by
-  oracle/Makefile) on top of the image's liblz4 1.9.4 / libzstd 1.5.5.
+  UNMODIFIED compression.c + storage.c (compiled from the pg_cryogen sources by
+  oracle/Makefile, PG_CRYOGEN_SRC) on top of the image's liblz4 1.9.4 / libzstd 1.5.5;
+  without it, the codec calls go to those two libraries directly.
 * ``oracle.port`` -- ctypes binding of ``oracle/libcryooracle.so``: our plain-C
   restatement of the LZ4 block format and the zstd frame format (RFC 8878).
 

@@ -22,14 +22,15 @@ def pytest_configure(config):
 
 @pytest.fixture(scope="session")
 def oracle_ref():
-    """The reference's own compression.c/storage.c on liblz4/libzstd (oracle/_ref)."""
+    """The reference's own compression.c/storage.c on liblz4/libzstd (oracle/_ref), built from the pg_cryogen
+    sources PG_CRYOGEN_SRC names or prebuilt.  Without it oracle.ref makes the codec calls on liblz4/libzstd
+    directly, and what needs the reference's storage.c is compared with its stored outputs (tests/golden)."""
     from oracle import ref
-    if not ref.available():
-        if os.path.exists("/root/reference/compression.c"):
-            subprocess.check_call(["make", "-s", "-C", os.path.join(ROOT, "oracle"), "ref"])
-        else:
-            pytest.fail("oracle/_ref/libcryoref.so missing and /root/reference absent")
-    ref.lib()
+    src = os.environ.get("PG_CRYOGEN_SRC", "")
+    if not ref.available() and src and os.path.exists(os.path.join(src, "compression.c")):
+        subprocess.check_call(["make", "-s", "-C", os.path.join(ROOT, "oracle"), "ref"])
+    if ref.available():
+        ref.lib()
     return ref
 
 

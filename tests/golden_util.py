@@ -33,3 +33,22 @@ def load():
 def plaintext(name: str) -> np.ndarray:
     key = name.rsplit("_", 1)[0]
     return PLAINTEXT[key]()
+
+
+def reference_outputs() -> dict:
+    """tests/golden/reference_outputs.json: what the reference's storage.c, storage.h and compression.c produced
+    (page layout, tuple walks, SHA-256 of built blocks, compressed sizes); README.md there says where from."""
+    import json
+    with open(os.path.join(HERE, "golden", "reference_outputs.json")) as f:
+        return json.load(f)
+
+
+def reference_block_sha256(oracle_ref, key: str, tuples) -> str:
+    """SHA-256 of the block the reference's storage.c builds from `tuples`: checked against the stored value
+    through oracle/_ref where it is present; the stored value is returned either way."""
+    import hashlib
+    want = reference_outputs()["block_sha256"][key]
+    if oracle_ref.available():
+        got = oracle_ref.build_block([bytes(t) for t in tuples])
+        assert hashlib.sha256(got.tobytes()).hexdigest() == want, key
+    return want

@@ -22,7 +22,8 @@ MiB = 1 << 20
 
 def test_reference_library_versions_are_the_pinned_ones(oracle_ref):
     assert oracle_ref.versions() == (10904, 10505)       # liblz4 1.9.4, libzstd 1.5.5
-    assert oracle_ref.guc_defaults() == (1, 1, 1)         # compression.c:16-18
+    if oracle_ref.available():                            # the reference's own GUC table (oracle/_ref)
+        assert oracle_ref.guc_defaults() == (1, 1, 1)     # compression.c:16-18
     assert oracle_ref.compress_bound(0) == 1052704        # LZ4_compressBound(1 MiB)
     assert oracle_ref.compress_bound(1) == 1052672        # ZSTD_compressBound(1 MiB)
 
@@ -35,6 +36,18 @@ def test_golden_streams_are_what_the_reference_writes(oracle_ref):
         assert np.array_equal(comp[0], stream), name
         out, ok = oracle_ref.decompress_one(method, stream)
         assert ok and np.array_equal(out, blk), name
+
+
+def test_compressed_sizes_are_what_the_reference_wrote(oracle_ref):
+    """Total compressed bytes of blocks 1000..1031 of each benchmark kind at lz4 acceleration 1 and zstd level 1,
+    as the reference wrote them in a recorded benchmark run (tests/golden/reference_outputs.json)."""
+    want = golden_util.reference_outputs()["compressed_bytes_blocks_1000_to_1031"]
+    assert len(want) == 12
+    for key, total in want.items():
+        kind, payload, codec = key.split("_")
+        blocks = bg.make_blocks(kind, payload, 1000, 32)
+        _, sizes, _ = oracle_ref.compress(0 if codec == "lz4a1" else 1, 1, blocks, nthreads=8, keep=False)
+        assert int(sizes.astype(np.int64).sum()) == total, key
 
 
 def test_port_decodes_golden_streams(oracle_port):

@@ -1,6 +1,6 @@
 """The page chain around the codec (SURVEY.md 8 f-1, a10), CPU part: the restatement of the reference's
 split (pg_cryogen.c:689-805) and gather (cache.c:100-176) in oracle/cryo_pages.c, pinned against the
-reference's own storage.h as compiled into oracle/_ref."""
+reference's own storage.h as compiled into oracle/_ref, and against its stored outputs (tests/golden)."""
 import ctypes as C
 
 import numpy as np
@@ -8,15 +8,21 @@ import numpy as np
 from oracle import pages as opg
 from pg_cryogen_b200 import blockgen as bg
 
+import golden_util
+
 PAGE = 8192
 
 
 def test_page_header_layout_is_the_references(oracle_ref):
-    """sizeof / offsetof from /root/reference/storage.h (compiled in oracle/_ref) = the restatement's."""
-    want = (C.c_uint32 * 12)()
-    oracle_ref.lib().oref_page_layout(want)
-    assert list(want) == opg.layout()
-    assert list(want)[:2] == [32, 48]           # SURVEY.md A.1: payload offsets 32 / 48
+    """sizeof / offsetof from the reference's storage.h (stored; compiled in oracle/_ref where present) = the
+    restatement's."""
+    want = golden_util.reference_outputs()["layout"]
+    if oracle_ref.available():
+        got = (C.c_uint32 * 12)()
+        oracle_ref.lib().oref_page_layout(got)
+        assert list(got) == want
+    assert want == opg.layout()
+    assert want[:2] == [32, 48]                 # SURVEY.md A.1: payload offsets 32 / 48
 
 
 def test_pages_needed_edges():
@@ -56,15 +62,21 @@ def test_split_then_gather_roundtrip_and_errors(oracle_ref):
 
 def test_tuple_walk_restatement_equals_the_references(oracle_ref):
     """cryo_oracle_block_tuple_stats against the loop of cryo_getnextslot around the reference's own
-    cryo_storage_fetch (oref_block_walk, compiled from /root/reference/storage.c)."""
-    L = oracle_ref.lib()
+    cryo_storage_fetch (oref_block_walk in oracle/_ref where present; its stored results)."""
+    stored = golden_util.reference_outputs()["tuple_walk"]
     for kind, pl, seed in (("S", "hex", 1), ("M", "lowcard", 2), ("D", "hex", 3), ("D", "random", 4)):
         b = bg.make_block(kind, pl, seed)
-        n, by = C.c_uint32(0), C.c_uint64(0)
-        L.oref_block_walk(C.c_void_p(b.ctypes.data), C.byref(n), C.byref(by))
-        assert opg.block_tuple_stats(b) == (n.value, by.value, 1), (kind, pl)
+        want = tuple(stored[f"{kind}_{pl}_{seed}"])
+        if oracle_ref.available():
+            n, by = C.c_uint32(0), C.c_uint64(0)
+            oracle_ref.lib().oref_block_walk(C.c_void_p(b.ctypes.data), C.byref(n), C.byref(by))
+            assert (n.value, by.value) == want, (kind, pl)
+        assert opg.block_tuple_stats(b) == (*want, 1), (kind, pl)
     empty = np.zeros(1 << 20, dtype=np.uint8)
-    L.oref_init_page(C.c_void_p(empty.ctypes.data))
+    if oracle_ref.available():
+        oracle_ref.lib().oref_init_page(C.c_void_p(empty.ctypes.data))
+    else:
+        empty[:8] = np.array([8, 1 << 20], dtype=np.uint32).view(np.uint8)      # cryo_init_page: lower, upper
     assert opg.block_tuple_stats(empty) == (0, 0, 1)
     bad = bg.make_block("S", "hex", 5).copy()
     bad[8 + 8 * 7: 8 + 8 * 7 + 4] = 0xFF                # item 8 points outside the block
