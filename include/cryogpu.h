@@ -283,6 +283,57 @@ int cryogpu_decompress_count_host(cryogpu_ctx *ctx, size_t n, const int32_t *met
                                   uint32_t *ntuples, uint64_t *tuple_bytes, int32_t *status);
 
 /*
+ * ------------------------------------------------------------ batched tuple fetch
+ *
+ * The random-read path (index fetch, bitmap heap scan, row lock, analyze: cryo_storage_fetch, storage.c:55-68):
+ * the tuples a caller names by TID (block, 1-based item position), packed, instead of whole decoded blocks.
+ *
+ *   item walk   as cryogpu_tuple_stats_device: ntuples = the largest cur with cur * 8 < lower; item p is the
+ *               CryoItemId {off, len} at byte 8 * p.  The table is valid iff lower >= 8, lower <= upper <=
+ *               block_size and every item lies inside [upper, block_size).
+ *   selection   sel_off == NULL: every item of every block in position order.  Else block i takes the positions
+ *               sel_pos[sel_off[i] .. sel_off[i + 1]) in that order; repeats are copied again; position 0 means
+ *               every item of the block (a lossy bitmap page).
+ *   output      the entries of all blocks in block order, then selection order.  Entry e: tup_off[e] (byte offset
+ *               into data, a multiple of 8: a HeapTupleHeader pointer into data is MAXALIGNed), tup_len[e] (the
+ *               item's len); the pad bytes up to MAXALIGN(len) are zero.  A position outside 1..ntuples gives
+ *               tup_off = UINT64_MAX, tup_len = 0 ("not found").  Block i's entries are
+ *               [block_first[i], block_first[i + 1]) (n + 1 values).
+ *   status[i]   the decoder's / chain check's status passes through (no entries); a decoded block whose item table
+ *               is invalid: CRYOGPU_ST_FORMAT (no entries).  Entries and bytes are placed by prefix sum over the
+ *               blocks; a block whose range would cross tup_cap or data_cap gets CRYOGPU_ST_OUTPUT and writes
+ *               nothing (its range stays reserved in block_first).
+ *   need[2]     {bytes, entries} the whole batch needs, whatever the capacities: size a retry with it.
+ *
+ * Bytes: read 8 + 8 * ntuples + the selected tuples per block; write sum MAXALIGN(len) + 12 per entry.
+ */
+
+/* Decoded blocks in HBM (block i at d_blocks + i * stride; d_blocks, stride 8-byte aligned; d_data 16-byte aligned).
+ * d_block_status (may be NULL): the decode's status[].  Enqueues work on `stream` only, like
+ * cryogpu_tuple_stats_device; calls on one context are ordered as the other device-resident calls are. */
+int cryogpu_tuples_device(cryogpu_ctx *ctx, size_t n, const uint8_t *d_blocks, uint64_t stride, uint32_t block_size,
+                          const int32_t *d_block_status, const uint64_t *d_sel_off, const uint32_t *d_sel_pos,
+                          uint8_t *d_data, uint64_t data_cap, uint64_t *d_tup_off, uint32_t *d_tup_len, uint64_t tup_cap,
+                          uint64_t *d_block_first, int32_t *d_status, uint64_t *d_need, void *stream);
+
+/* Compressed streams in host memory in, tuples out: csize in, the tuples and per-block metadata back.  Synchronous;
+ * large batches go in chunks (offsets are global); pinned data / tup_off / tup_len are written straight by the
+ * copies.  cryogpu_last_transfer_bytes reports the bytes moved. */
+int cryogpu_decompress_tuples_host(cryogpu_ctx *ctx, size_t n, const int32_t *methods, const void *const *src,
+                                   const uint32_t *src_size, uint32_t block_size, const uint64_t *sel_off,
+                                   const uint32_t *sel_pos, void *data, uint64_t data_cap, uint64_t *tup_off,
+                                   uint32_t *tup_len, uint64_t tup_cap, uint64_t *block_first, int32_t *status,
+                                   uint64_t *need);
+
+/* Page chains in (as cryogpu_decompress_pages_host describes them), tuples out; methods[i] / comp_size[i] (may be
+ * NULL): compression_method and compressed_size of the first page's header. */
+int cryogpu_decompress_pages_tuples_host(cryogpu_ctx *ctx, size_t n, const void *const *pages, const uint32_t *page_blkno,
+                                         const uint32_t *chain_off, uint32_t block_size, const uint64_t *sel_off,
+                                         const uint32_t *sel_pos, void *data, uint64_t data_cap, uint64_t *tup_off,
+                                         uint32_t *tup_len, uint64_t tup_cap, uint64_t *block_first, int32_t *status,
+                                         int32_t *methods, uint32_t *comp_size, uint64_t *need);
+
+/*
  * Multi-GPU host variants: the batch is split into contiguous block ranges, one
  * per context (one host thread + stream per GPU, no collective; SURVEY.md 8(e)).
  */

@@ -78,6 +78,16 @@ _PROTOS = {
                                              C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "cryogpu_decompress_count_host": (C.c_int, [C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32,
                                                 C.c_void_p, C.c_void_p, C.c_void_p]),
+    "cryogpu_tuples_device": (C.c_int, [C.c_void_p, C.c_size_t, C.c_void_p, C.c_uint64, C.c_uint32, C.c_void_p, C.c_void_p,
+                                        C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p,
+                                        C.c_void_p, C.c_void_p, C.c_void_p]),
+    "cryogpu_decompress_tuples_host": (C.c_int, [C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32,
+                                                 C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p,
+                                                 C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "cryogpu_decompress_pages_tuples_host": (C.c_int, [C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32,
+                                                       C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p,
+                                                       C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p,
+                                                       C.c_void_p, C.c_void_p]),
     "cryogpu_decompress_host_multi": (C.c_int, [C.c_void_p, C.c_int, C.c_size_t, C.c_void_p,
                                                 C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32,
                                                 C.c_void_p, C.c_void_p]),
@@ -290,6 +300,80 @@ class CryoGPU:
             self.handle, n, method, level_or_accel, srcp, block_size, blknos.ctypes.data, cap, created_xid, outp,
             npg.ctypes.data, csz.ctypes.data, st.ctypes.data), "cryogpu_compress_pages_host")
         return npg, csz, st
+
+
+    # ---- batched tuple fetch (cryo_storage_fetch, storage.c:55-68, for many TIDs at once) ----
+
+    def tuples_device(self, blocks, stride, n: int, block_status, sel_off, sel_pos, data, data_cap: int, tup_off, tup_len,
+                      tup_cap: int, block_first, status, need, block_size: int = CRYO_BLCKSZ, stream: int | None = None):
+        """Decoded blocks in HBM -> packed tuples (torch CUDA tensors or device pointers); only enqueues."""
+        self._check(self.lib.cryogpu_tuples_device(
+            self.handle, n, _ptr(blocks), stride, block_size, _ptr(block_status), _ptr(sel_off), _ptr(sel_pos), _ptr(data),
+            data_cap, _ptr(tup_off), _ptr(tup_len), tup_cap, _ptr(block_first), _ptr(status), _ptr(need),
+            _stream(stream)), "cryogpu_tuples_device")
+
+    def _tuples_host(self, call, what, n, sel, data_cap, tup_cap):
+        """Runs call(sel_off, sel_pos, data, data_cap, tup_off, tup_len, tup_cap, block_first, status, need); with a
+        capacity of None it first asks for what the batch needs (a call with no room), then fetches."""
+        sel_off, sel_pos = _sel_arrays(sel, n)
+        bf = np.zeros(n + 1, dtype=np.uint64)
+        st = np.full(n, -1, dtype=np.int32)
+        need = np.zeros(2, dtype=np.uint64)
+        if data_cap is None or tup_cap is None:
+            self._check(call(_ptr(sel_off), _ptr(sel_pos), None, 0, None, None, 0, bf.ctypes.data, st.ctypes.data,
+                             need.ctypes.data), what)
+            data_cap = int(need[0]) if data_cap is None else data_cap
+            tup_cap = int(need[1]) if tup_cap is None else tup_cap
+        data = np.zeros(max(data_cap, 1), dtype=np.uint8)
+        to = np.zeros(max(tup_cap, 1), dtype=np.uint64)
+        tl = np.zeros(max(tup_cap, 1), dtype=np.uint32)
+        self._check(call(_ptr(sel_off), _ptr(sel_pos), data.ctypes.data, data_cap, to.ctypes.data, tl.ctypes.data, tup_cap,
+                         bf.ctypes.data, st.ctypes.data, need.ctypes.data), what)
+        return data[:data_cap], to[:tup_cap], tl[:tup_cap], bf, st, (int(need[0]), int(need[1]))
+
+    def decompress_tuples_host(self, methods, chunks, sel=None, block_size: int = CRYO_BLCKSZ, data_cap: int | None = None,
+                               tup_cap: int | None = None):
+        """Compressed blocks in, tuples out.  sel: None (every item) or per block a list of positions (0 = every item).
+        Returns (data, tup_off, tup_len, block_first, status, (bytes, entries) needed)."""
+        n = len(chunks)
+        chunks = [np.ascontiguousarray(c, dtype=np.uint8) for c in chunks]
+        methods = np.ascontiguousarray(np.broadcast_to(np.asarray(methods, dtype=np.int32), (n,)))
+        sizes = np.array([c.size for c in chunks], dtype=np.uint32)
+        srcp = (C.c_void_p * max(n, 1))(*[c.ctypes.data for c in chunks])
+
+        def call(*a):
+            return self.lib.cryogpu_decompress_tuples_host(self.handle, n, methods.ctypes.data, srcp, sizes.ctypes.data,
+                                                           block_size, *a)
+        return self._tuples_host(call, "cryogpu_decompress_tuples_host", n, sel, data_cap, tup_cap)
+
+    def decompress_pages_tuples_host(self, relation: np.ndarray, chains, sel=None, block_size: int = CRYO_BLCKSZ,
+                                     data_cap: int | None = None, tup_cap: int | None = None):
+        """Page chains (as decompress_pages_host takes them) in, tuples out.  Returns (data, tup_off, tup_len,
+        block_first, status, need, methods, comp_size)."""
+        n = len(chains)
+        flat = [b for ch in chains for b in ch]
+        coff = np.zeros(n + 1, dtype=np.uint32)
+        coff[1:] = np.cumsum([len(ch) for ch in chains])
+        blk = np.asarray(flat + [0], dtype=np.uint32)
+        pagep = (C.c_void_p * max(len(flat), 1))(*[relation[b].ctypes.data for b in flat])
+        me = np.full(n, -1, dtype=np.int32)
+        csz = np.zeros(n, dtype=np.uint32)
+
+        def call(so, sp, data, dcap, to, tl, tcap, bf, st, need):
+            return self.lib.cryogpu_decompress_pages_tuples_host(self.handle, n, pagep, blk.ctypes.data, coff.ctypes.data,
+                                                                 block_size, so, sp, data, dcap, to, tl, tcap, bf, st,
+                                                                 me.ctypes.data, csz.ctypes.data, need)
+        return self._tuples_host(call, "cryogpu_decompress_pages_tuples_host", n, sel, data_cap, tup_cap) + (me, csz)
+
+
+def _sel_arrays(sel, n: int):
+    """Per-block position lists (None: every item) -> (sel_off uint64 [n + 1], sel_pos uint32) or (None, None)."""
+    if sel is None:
+        return None, None
+    assert len(sel) == n
+    off = np.zeros(n + 1, dtype=np.uint64)
+    off[1:] = np.cumsum([len(s) for s in sel])
+    return off, np.array([p for s in sel for p in s] + [0], dtype=np.uint32)
 
 
 def pages_needed(compressed_size: int) -> int:

@@ -1,0 +1,363 @@
+/*
+ * cryo_tuples.cuh -- batched tuple fetch from decoded cryo blocks in HBM: the random-read path of the reference
+ * (index fetch, bitmap heap scan, row lock, analyze: cryo_storage_fetch, storage.c:55-68, reached through
+ * pg_cryogen.c:377-463, :862-895, :987-1034).  The caller names tuples by item position; only the selected tuples
+ * cross the bus, packed, instead of whole 1 MiB blocks.
+ *
+ *   select  one warp per block: the item walk of k_tuple_stats (ntuples = the largest cur with cur * 8 < lower;
+ *           item p is the CryoItemId {off, len} at byte 8 * p), the table's validity (lower >= 8,
+ *           lower <= upper <= block_size, every item inside [upper, block_size)), and the selection: every item,
+ *           or the caller's positions in the caller's order (repeats allowed; 0 = every item of the block).  Out:
+ *           the block's entry count and its packed bytes (sum of MAXALIGN(len) over the entries).
+ *   scan    one CTA: exclusive prefix sums of (entries, bytes) over the batch -> block_first[], the byte start of
+ *           every block, the two totals; a block whose range would cross tup_cap or data_cap is CRYOGPU_ST_OUTPUT.
+ *   gather  one warp per block walks the selection again: per group of 32 entries a warp scan places them, a
+ *           tuple longer than TUP_LARGE is copied by the whole warp, shorter ones by 8-lane groups (an S tuple is
+ *           61 bytes).  Reads touch the item table and the selected tuples only.
+ *
+ * Output: tuples start on 8-byte boundaries (a HeapTupleHeader pointer into the buffer is MAXALIGNed); the pad
+ * bytes up to MAXALIGN(len) are zero.  A position outside 1..ntuples gives tup_off = TUP_NONE, tup_len = 0.
+ * Blocks are 8-byte aligned (stride too); the data buffer is 16-byte aligned.
+ */
+#pragma once
+#include "cryo_common.cuh"
+
+#define TUP_NONE        0xFFFFFFFFFFFFFFFFull   /* tup_off of a position that does not exist */
+#define TUP_MISSING     0xFFFFFFFFu             /* internal: no item behind the position */
+#define TUP_LARGE       128u                    /* longer tuples: one warp each; shorter: one 8-lane group each */
+#define TUP_SCAN_THREADS 256u
+#define TUP_SCAN_ITEMS  4u                      /* blocks per thread and tile of the scan */
+
+typedef unsigned long long tup_u64;
+
+CRYO_DEV tup_u64 tup_ld8(const uint8_t *p) { return *reinterpret_cast<const tup_u64 *>(p); }
+CRYO_DEV void tup_st8(uint8_t *p, tup_u64 v) { *reinterpret_cast<tup_u64 *>(p) = v; }
+CRYO_DEV uint32_t tup_maxalign(uint32_t len) { return (len + 7u) & ~7u; }
+
+/* number of items, as k_tuple_stats counts them (block_size >= 16) */
+CRYO_DEV uint32_t tup_count(const uint8_t *block, uint32_t block_size)
+{
+    const uint32_t lower = ld4(block);
+    uint32_t n = lower ? (lower - 1u) / 8u : 0u;
+
+    if ((tup_u64) n * 8u + 8u > block_size)
+        n = block_size / 8u - 1u;
+    return n;
+}
+
+CRYO_DEV uint2 tup_item(const uint8_t *block, uint32_t p)
+{
+    return *reinterpret_cast<const uint2 *>(block + 8u * p);
+}
+
+/*
+ * Select, one warp, one block.  in_status: the decoder's / chain check's outcome (a failed block keeps it and gets
+ * no entries).  sel_off == NULL: every item; else the positions sel_pos[sel_off[b] .. sel_off[b + 1]).
+ */
+CRYO_DEV void tup_select_block(const uint8_t *block, uint32_t block_size, int32_t in_status, const tup_u64 *sel_off,
+                               const uint32_t *sel_pos, uint32_t b, tup_u64 *cnt, tup_u64 *bytes, int32_t *status,
+                               uint32_t lane)
+{
+    int32_t st = in_status;
+    tup_u64 c = 0, by = 0;
+
+    if (st == ST_OK)
+    {
+        const uint32_t lower = ld4(block), upper = ld4(block + 4), n = tup_count(block, block_size);
+        bool ok = lower >= 8u && lower <= upper && upper <= block_size;
+        tup_u64 all = 0;
+
+        for (uint32_t cur = 1u + lane; ok && cur <= n; cur += 32u)
+        {
+            const uint2 it = tup_item(block, cur);
+
+            all += tup_maxalign(it.y);
+            if (it.x < upper || it.x > block_size || it.y > block_size - it.x)
+                ok = false;
+        }
+        ok = __all_sync(CRYO_FULL, ok);
+#pragma unroll
+        for (uint32_t d = 16; d; d >>= 1)
+            all += __shfl_xor_sync(CRYO_FULL, all, d);
+        if (!ok)
+            st = ST_FORMAT;
+        else if (!sel_off)
+        {
+            c = n;
+            by = all;
+        }
+        else
+        {
+            for (tup_u64 i = sel_off[b] + lane; i < sel_off[b + 1]; i += 32u)
+            {
+                const uint32_t p = sel_pos[i];
+
+                c += p == 0 ? n : 1u;
+                by += p == 0 ? all : p <= n ? tup_maxalign(tup_item(block, p).y) : 0u;
+            }
+#pragma unroll
+            for (uint32_t d = 16; d; d >>= 1)
+            {
+                c += __shfl_xor_sync(CRYO_FULL, c, d);
+                by += __shfl_xor_sync(CRYO_FULL, by, d);
+            }
+        }
+    }
+    if (lane == 0)
+    {
+        *cnt = st == ST_OK ? c : 0u;
+        *bytes = st == ST_OK ? by : 0u;
+        *status = st;
+    }
+}
+
+/*
+ * Scan, one CTA of nthr threads (a multiple of 32, at most 32 warps).  ent0 / byte0: where this batch starts in the
+ * caller's output (the host calls cut a batch into chunks); tup_cap / data_cap: the caller's capacities, global.
+ * block_first[n + 1] and byte_first[n + 1] are global; need = {bytes, entries} of this batch.  smem: 2 x 32 words.
+ */
+CRYO_DEV void tup_scan(uint32_t n, const tup_u64 *cnt, const tup_u64 *bytes, int32_t *status, tup_u64 ent0, tup_u64 byte0,
+                       tup_u64 tup_cap, tup_u64 data_cap, tup_u64 *block_first, tup_u64 *byte_first, tup_u64 *need,
+                       tup_u64 *smem, uint32_t tid, uint32_t nthr)
+{
+    const uint32_t lane = tid & 31u, w = tid >> 5, nw = nthr >> 5;
+    tup_u64 carry_e = 0, carry_b = 0;
+
+    for (uint32_t base = 0; base < n; base += nthr * TUP_SCAN_ITEMS)
+    {
+        const uint32_t i0 = base + tid * TUP_SCAN_ITEMS;
+        tup_u64 le = 0, lb = 0;
+
+        for (uint32_t k = 0; k < TUP_SCAN_ITEMS; k++)
+            if (i0 + k < n)
+            {
+                le += cnt[i0 + k];
+                lb += bytes[i0 + k];
+            }
+        tup_u64 xe = le, xb = lb;
+
+        for (uint32_t d = 1; d < 32u; d <<= 1)
+        {
+            const tup_u64 ye = __shfl_up_sync(CRYO_FULL, xe, d), yb = __shfl_up_sync(CRYO_FULL, xb, d);
+
+            if (lane >= d)
+            {
+                xe += ye;
+                xb += yb;
+            }
+        }
+        if (lane == 31u)
+        {
+            smem[2 * w] = xe;
+            smem[2 * w + 1] = xb;
+        }
+        __syncthreads();
+        tup_u64 pe = carry_e, pb = carry_b, te = 0, tb = 0;
+
+        for (uint32_t k = 0; k < nw; k++)
+        {
+            if (k < w)
+            {
+                pe += smem[2 * k];
+                pb += smem[2 * k + 1];
+            }
+            te += smem[2 * k];
+            tb += smem[2 * k + 1];
+        }
+        pe += xe - le;
+        pb += xb - lb;
+        for (uint32_t k = 0; k < TUP_SCAN_ITEMS; k++)
+            if (i0 + k < n)
+            {
+                const uint32_t i = i0 + k;
+                const tup_u64 e = ent0 + pe, by = byte0 + pb;
+
+                block_first[i] = e;
+                byte_first[i] = by;
+                if (status[i] == ST_OK && cnt[i] && (e + cnt[i] > tup_cap || by + bytes[i] > data_cap))
+                    status[i] = ST_OUTPUT;
+                pe += cnt[i];
+                pb += bytes[i];
+            }
+        carry_e += te;
+        carry_b += tb;
+        __syncthreads();
+    }
+    if (tid == 0)
+    {
+        block_first[n] = ent0 + carry_e;
+        byte_first[n] = byte0 + carry_b;
+        need[0] = carry_b;
+        need[1] = carry_e;
+    }
+}
+
+/*
+ * Word k (bytes [8k, 8k + 8)) of the len-byte tuple at src, zero past len.  src has any alignment: the word is put
+ * together from the aligned 8-byte words around it (the second only when it holds tuple bytes).
+ */
+CRYO_DEV tup_u64 tup_word(const uint8_t *src, uint32_t len, uint32_t k)
+{
+    const uint32_t sh = (uint32_t) ((uintptr_t) src & 7u), left = len - 8u * k;
+    const uint8_t *a = src - sh + 8u * k;
+    tup_u64 w = tup_ld8(a) >> (8u * sh);
+
+    if (sh && 8u * k + 8u - sh < len)
+        w |= tup_ld8(a + 8u) << (64u - 8u * sh);
+    if (left < 8u)
+        w &= (1ull << (8u * left)) - 1ull;
+    return w;
+}
+
+/*
+ * The tuple at src (any alignment) to dst (8-byte aligned), zero-padded to MAXALIGN(len), by a team of nt threads.
+ * Where src and dst agree mod 16 the body moves as 16-byte vectors; otherwise (and at the ends) as aligned 8-byte
+ * words, each shifted together from two aligned loads.
+ */
+CRYO_DEV void tup_copy(uint8_t *dst, const uint8_t *src, uint32_t len, uint32_t t, uint32_t nt)
+{
+    const uint32_t nw = (len + 7u) / 8u;
+    uint32_t k0 = 0;
+
+    if ((((uintptr_t) src ^ (uintptr_t) dst) & 15u) == 0)
+    {
+        const uint32_t h = ((uintptr_t) dst & 8u) ? 1u : 0u;     /* one word up to the first 16-byte boundary */
+        const uint32_t nv = len >= 8u * h ? (len - 8u * h) / 16u : 0u;
+
+        if (nv)
+        {
+            if (h && t == 0)
+                tup_st8(dst, tup_ld8(src));
+            for (uint32_t v = t; v < nv; v += nt)
+                st16(dst + 8u * h + 16u * v, ld16(src + 8u * h + 16u * v));
+            k0 = h + 2u * nv;
+        }
+    }
+    for (uint32_t k = k0 + t; k < nw; k += nt)
+        tup_st8(dst + 8u * k, tup_word(src, len, k));
+}
+
+/* Output pointers of the gather: entries / bytes are global; the arrays start at entry ent0 and byte byte0. */
+struct TupOut
+{
+    uint8_t  *data;
+    tup_u64  *tup_off;
+    uint32_t *tup_len;
+    tup_u64   ent0, byte0;
+};
+
+/*
+ * One group of up to 32 entries, one per lane with act set, in lane order: so = the tuple's offset in the block
+ * (TUP_MISSING: the position does not exist), len its length.  ent / boff: the next entry and byte, advanced.
+ */
+CRYO_DEV void tup_emit(bool act, uint32_t so, uint32_t len, const uint8_t *block, tup_u64 &ent, tup_u64 &boff,
+                       TupOut o, uint32_t lane)
+{
+    const bool found = act && so != TUP_MISSING;
+    const uint32_t sz = found ? tup_maxalign(len) : 0u;
+    tup_u64 x = sz;
+
+    for (uint32_t d = 1; d < 32u; d <<= 1)
+    {
+        const tup_u64 y = __shfl_up_sync(CRYO_FULL, x, d);
+
+        if (lane >= d)
+            x += y;
+    }
+    const tup_u64 total = __shfl_sync(CRYO_FULL, x, 31);
+    const unsigned am = __ballot_sync(CRYO_FULL, act);
+    const tup_u64 my = boff + x - sz;
+
+    if (act)
+    {
+        const tup_u64 e = ent + (uint32_t) __popc(am & ((1u << lane) - 1u)) - o.ent0;
+
+        o.tup_off[e] = found ? my : TUP_NONE;
+        o.tup_len[e] = found ? len : 0u;
+    }
+    const bool big = found && len > TUP_LARGE, small = found && !big;
+    unsigned bm = __ballot_sync(CRYO_FULL, big);
+
+    while (bm)
+    {
+        const int l = __ffs((int) bm) - 1;
+        const uint32_t ls = __shfl_sync(CRYO_FULL, so, l), ll = __shfl_sync(CRYO_FULL, len, l);
+        const tup_u64 lo = __shfl_sync(CRYO_FULL, my, l);
+
+        bm &= bm - 1u;
+        tup_copy(o.data + (lo - o.byte0), block + ls, ll, lane, 32u);
+    }
+    if (__any_sync(CRYO_FULL, small))
+    {
+        const uint32_t g = lane >> 3;
+
+        for (uint32_t j = 0; j < 8u; j++)
+        {
+            const int src = (int) (4u * j + g);
+            const int sm = __shfl_sync(CRYO_FULL, small ? 1 : 0, src);
+            const uint32_t ls = __shfl_sync(CRYO_FULL, so, src), ll = __shfl_sync(CRYO_FULL, len, src);
+            const tup_u64 lo = __shfl_sync(CRYO_FULL, my, src);
+
+            if (sm)
+                tup_copy(o.data + (lo - o.byte0), block + ls, ll, lane & 7u, 8u);
+        }
+    }
+    ent += (uint32_t) __popc(am);
+    boff += total;
+}
+
+/* every item of the block, in position order */
+CRYO_DEV void tup_emit_all(const uint8_t *block, uint32_t n, tup_u64 &ent, tup_u64 &boff, TupOut o, uint32_t lane)
+{
+    for (uint32_t c0 = 0; c0 < n; c0 += 32u)
+    {
+        const uint32_t cur = c0 + 1u + lane;
+        const bool act = cur <= n;
+        const uint2 it = act ? tup_item(block, cur) : make_uint2(0u, 0u);
+
+        tup_emit(act, it.x, it.y, block, ent, boff, o, lane);
+    }
+}
+
+/*
+ * Gather, one warp, one block whose status after the scan is CRYOGPU_ST_OK.  ent / boff: the block's first entry
+ * and byte (block_first[b], the scan's byte start).
+ */
+CRYO_DEV void tup_gather_block(const uint8_t *block, uint32_t block_size, const tup_u64 *sel_off, const uint32_t *sel_pos,
+                               uint32_t b, tup_u64 ent, tup_u64 boff, TupOut o, uint32_t lane)
+{
+    const uint32_t n = tup_count(block, block_size);
+    /* every item: a selection of one position 0 */
+    const tup_u64 s0 = sel_off ? sel_off[b] : 0u, s1 = sel_off ? sel_off[b + 1] : 1u;
+
+    for (tup_u64 i0 = s0; i0 < s1; i0 += 32u)
+    {
+        const bool have = i0 + lane < s1;
+        const uint32_t p = !have ? 1u : sel_off ? sel_pos[i0 + lane] : 0u;
+        unsigned zm = __ballot_sync(CRYO_FULL, have && p == 0);
+        uint32_t cur = 0;
+
+        /* runs of single positions, each followed by at most one 0 (every item) */
+        for (;;)
+        {
+            const uint32_t z = zm ? (uint32_t) (__ffs((int) zm) - 1) : 32u;
+            const bool act = have && lane >= cur && lane < z;
+            uint32_t so = TUP_MISSING, len = 0;
+
+            if (act && p >= 1u && p <= n)
+            {
+                const uint2 it = tup_item(block, p);
+
+                so = it.x;
+                len = it.y;
+            }
+            if (__any_sync(CRYO_FULL, act))
+                tup_emit(act, so, len, block, ent, boff, o, lane);
+            if (z == 32u)
+                break;
+            tup_emit_all(block, n, ent, boff, o, lane);
+            zm &= zm - 1u;
+            cur = z + 1u;
+        }
+    }
+}

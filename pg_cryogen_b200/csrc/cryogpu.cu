@@ -16,6 +16,7 @@
 #include "lz4_encode.cuh"
 #include "zstd_encode.cuh"
 #include "cryo_pages.cuh"
+#include "cryo_tuples.cuh"
 
 #include <cuda_runtime.h>
 
@@ -869,6 +870,36 @@ k_tuple_stats(const uint8_t *blocks, uint64_t stride, uint32_t block_size, const
     pg_tuple_stats(blocks + b * stride, block_size, ntuples + b, tuple_bytes + b, valid + b, lane);
 }
 
+/* batched tuple fetch (cryo_tuples.cuh): select and gather one warp per block, 8 blocks per CTA; the scan one CTA */
+__global__ void __launch_bounds__(256)
+k_tuple_select(const uint8_t *blocks, uint64_t stride, uint32_t block_size, const int32_t *block_status,
+               const tup_u64 *sel_off, const uint32_t *sel_pos, tup_u64 *cnt, tup_u64 *bytes, int32_t *status, uint32_t n)
+{
+    const uint32_t b = blockIdx.x * 8u + (threadIdx.x >> 5), lane = threadIdx.x & 31u;
+
+    if (b < n)
+        tup_select_block(blocks + b * stride, block_size, block_status ? block_status[b] : ST_OK, sel_off, sel_pos, b,
+                         cnt + b, bytes + b, status + b, lane);
+}
+
+__global__ void __launch_bounds__(TUP_SCAN_THREADS)
+k_tuple_scan(uint32_t n, const tup_u64 *cnt, const tup_u64 *bytes, int32_t *status, tup_u64 ent0, tup_u64 byte0,
+             tup_u64 tup_cap, tup_u64 data_cap, tup_u64 *block_first, tup_u64 *byte_first, tup_u64 *need)
+{
+    tup_scan(n, cnt, bytes, status, ent0, byte0, tup_cap, data_cap, block_first, byte_first, need,
+             (tup_u64 *) CRYO_SMEM_BASE(), threadIdx.x, TUP_SCAN_THREADS);
+}
+
+__global__ void __launch_bounds__(256, 4)      /* 4 CTAs per SM: 62 registers, no spills (a bare 256 spilled) */
+k_tuple_gather(const uint8_t *blocks, uint64_t stride, uint32_t block_size, const int32_t *status, const tup_u64 *sel_off,
+               const uint32_t *sel_pos, const tup_u64 *block_first, const tup_u64 *byte_first, TupOut o, uint32_t n)
+{
+    const uint32_t b = blockIdx.x * 8u + (threadIdx.x >> 5), lane = threadIdx.x & 31u;
+
+    if (b < n && status[b] == ST_OK)
+        tup_gather_block(blocks + b * stride, block_size, sel_off, sel_pos, b, block_first[b], byte_first[b], o, lane);
+}
+
 /* CRYOGPU_LZ4_KERNEL = warp | cx forces one LZ4 decoder for every block; default: routed per block */
 static int
 lz4_kernel_choice()
@@ -1310,6 +1341,8 @@ struct cryogpu_ctx
     DevBuf       zp[2];                 /* zstd pipeline work areas (zstd_decode_p.cuh), per lane */
     DevBuf       lzw[2];                /* CTA-per-block LZ4 decoder work areas (lz4c_bytes), per lane */
     DevBuf       pgw;                   /* page-chain calls: gathered streams / compressed blocks before the split */
+    DevBuf       tpw, tpo;              /* tuple fetch: per-block counts and offsets, selection; packed output (host calls) */
+    DevBuf       h_tpw, h_tpo;          /* tuple fetch, host calls: pinned selection / results, packed output */
     cudaEvent_t  busy = nullptr;        /* end of the last device-resident call: the work areas are shared */
     cudaStream_t zaux[2][2] = {{nullptr, nullptr}, {nullptr, nullptr}};   /* side streams of the pipeline's concurrent stages */
     cudaEvent_t  zev[2][4] = {{nullptr, nullptr, nullptr, nullptr}, {nullptr, nullptr, nullptr, nullptr}};
@@ -1543,6 +1576,10 @@ cryogpu_shutdown(cryogpu_ctx *ctx)
     cudaFree(ctx->lzw[0].p);
     cudaFree(ctx->lzw[1].p);
     cudaFree(ctx->pgw.p);
+    cudaFree(ctx->tpw.p);
+    cudaFree(ctx->tpo.p);
+    cudaFreeHost(ctx->h_tpw.p);
+    cudaFreeHost(ctx->h_tpo.p);
     if (ctx->busy)
         cudaEventDestroy(ctx->busy);
     cudaFree(ctx->predef);
@@ -2417,6 +2454,354 @@ cryogpu_decompress_count_host(cryogpu_ctx *ctx, size_t n, const int32_t *methods
             if (status[lo + i] == CRYOGPU_ST_OK && !h_ok[i])
                 status[lo + i] = CRYOGPU_ST_FORMAT;
     }
+    ctx->last_h2d = h2d;
+    ctx->last_d2h = d2h;
+    return CRYOGPU_OK;
+}
+
+/* ------------------------------------------------------- batched tuple fetch */
+
+static size_t
+tp_al(size_t v)
+{
+    return (v + 255) & ~(size_t) 255;
+}
+
+/*
+ * Select and scan of one batch on st (ctx->mu held, st ordered after ctx->busy).  work: 4n + 4 words of the context's
+ * tuple area: cnt[n] | bytes[n] | byte_first[n + 1] | (room for block_first[n + 1] and need[2] of the host calls).
+ */
+static int
+tuples_place(cudaStream_t st, size_t n, const uint8_t *d_blocks, uint64_t stride, uint32_t block_size,
+             const int32_t *d_block_status, const tup_u64 *d_sel_off, const uint32_t *d_sel_pos, uint64_t ent0, uint64_t byte0,
+             uint64_t data_cap, uint64_t tup_cap, tup_u64 *d_block_first, int32_t *d_status, tup_u64 *d_need, tup_u64 *work)
+{
+    if (n)
+        k_tuple_select<<<(unsigned) ((n + 7) / 8), 256, 0, st>>>(d_blocks, stride, block_size, d_block_status, d_sel_off,
+                                                                 d_sel_pos, work, work + n, d_status, (uint32_t) n);
+    k_tuple_scan<<<1, TUP_SCAN_THREADS, 64 * sizeof(tup_u64), st>>>((uint32_t) n, work, work + n, d_status, ent0, byte0, tup_cap,
+                                                                    data_cap, d_block_first, work + 2 * n, d_need);
+    CU(cudaGetLastError());
+    return CRYOGPU_OK;
+}
+
+static int
+tuples_gather(cudaStream_t st, size_t n, const uint8_t *d_blocks, uint64_t stride, uint32_t block_size, const int32_t *d_status,
+              const tup_u64 *d_sel_off, const uint32_t *d_sel_pos, const tup_u64 *d_block_first, const tup_u64 *work, TupOut o)
+{
+    if (n)
+        k_tuple_gather<<<(unsigned) ((n + 7) / 8), 256, 0, st>>>(d_blocks, stride, block_size, d_status, d_sel_off, d_sel_pos,
+                                                                 d_block_first, work + 2 * n, o, (uint32_t) n);
+    CU(cudaGetLastError());
+    return CRYOGPU_OK;
+}
+
+extern "C" int
+cryogpu_tuples_device(cryogpu_ctx *ctx, size_t n, const uint8_t *d_blocks, uint64_t stride, uint32_t block_size,
+                      const int32_t *d_block_status, const uint64_t *d_sel_off, const uint32_t *d_sel_pos, uint8_t *d_data,
+                      uint64_t data_cap, uint64_t *d_tup_off, uint32_t *d_tup_len, uint64_t tup_cap, uint64_t *d_block_first,
+                      int32_t *d_status, uint64_t *d_need, void *stream)
+{
+    if (!ctx)
+        return fail(CRYOGPU_E_ARG, "ctx is NULL");
+    if (!d_blocks || !d_block_first || !d_status || !d_need || (d_sel_off && !d_sel_pos) || (data_cap && !d_data) ||
+        (tup_cap && (!d_tup_off || !d_tup_len)))
+        return fail(CRYOGPU_E_ARG, "NULL device pointer");
+    if (((uintptr_t) d_blocks & 7) || (stride & 7) || block_size < 16 || block_size > (1u << 27) || stride < block_size ||
+        ((uintptr_t) d_data & 15) || ((uintptr_t) d_tup_off & 7) || ((uintptr_t) d_block_first & 7) ||
+        ((uintptr_t) d_sel_off & 7) || ((uintptr_t) d_need & 7) || n > 0x7fffffffu)
+        return fail(CRYOGPU_E_ARG, "blocks, stride, block_first, sel_off, tup_off 8-byte aligned, data 16-byte aligned, "
+                                   "16 <= block_size <= stride");
+    cudaStream_t st = stream ? (cudaStream_t) stream : ctx->stream;
+
+    CU(cudaSetDevice(ctx->device));
+    std::lock_guard<std::recursive_mutex> g(ctx->mu);
+
+    CU(cudaStreamWaitEvent(st, ctx->busy, 0));
+    int rc = dev_reserve(ctx->tpw, (4 * n + 4) * sizeof(tup_u64));
+
+    if (rc != CRYOGPU_OK)
+        return rc;
+    tup_u64 *work = (tup_u64 *) ctx->tpw.p;
+    const TupOut o = {d_data, (tup_u64 *) d_tup_off, d_tup_len, 0, 0};
+
+    if ((rc = tuples_place(st, n, d_blocks, stride, block_size, d_block_status, (const tup_u64 *) d_sel_off, d_sel_pos, 0, 0,
+                           data_cap, tup_cap, (tup_u64 *) d_block_first, d_status, (tup_u64 *) d_need, work)) != CRYOGPU_OK ||
+        (rc = tuples_gather(st, n, d_blocks, stride, block_size, d_status, (const tup_u64 *) d_sel_off, d_sel_pos,
+                            (const tup_u64 *) d_block_first, work, o)) != CRYOGPU_OK)
+        return rc;
+    CU(cudaEventRecord(ctx->busy, st));
+    return CRYOGPU_OK;
+}
+
+/*
+ * Tuple fetch of one chunk of a host call, blocks [lo, lo + cnt), decoded into d_blocks with their statuses in d_st by
+ * work already enqueued on ctx->stream (ctx->mu held).  Entries and bytes continue from ent_base / byte_base, which
+ * advance by what the chunk needs.  Two round trips: the placement (so that only the bytes that fit are staged and
+ * copied), then the packed tuples, straight into the caller's buffers when they are pinned.
+ */
+static int
+tuples_chunk_host(cryogpu_ctx *ctx, size_t lo, size_t cnt, const uint8_t *d_blocks, uint64_t stride, uint32_t block_size,
+                  int32_t *d_st, const uint64_t *sel_off, const uint32_t *sel_pos, void *data, uint64_t data_cap,
+                  uint64_t *tup_off, uint32_t *tup_len, uint64_t tup_cap, uint64_t *block_first, int32_t *status,
+                  uint64_t &ent_base, uint64_t &byte_base, uint64_t &h2d, uint64_t &d2h)
+{
+    const size_t m = sel_off ? (size_t) (sel_off[lo + cnt] - sel_off[lo]) : 0;
+    const size_t work_bytes = tp_al((4 * cnt + 4) * 8), sel_bytes = sel_off ? tp_al((cnt + 1) * 8) + tp_al(m * 4 + 4) : 0;
+    const size_t meta_words = 2 * (cnt + 1) + 2;        /* byte_first | block_first | need */
+    int          rc;
+
+    if ((rc = dev_reserve(ctx->tpw, work_bytes + sel_bytes)) != CRYOGPU_OK ||
+        (rc = host_reserve(ctx->h_tpw, sel_bytes + meta_words * 8 + cnt * 4)) != CRYOGPU_OK)
+        return rc;
+    tup_u64 *work = (tup_u64 *) ctx->tpw.p, *d_sel_off = nullptr;
+    uint32_t *d_sel_pos = nullptr;
+    uint8_t  *hw = (uint8_t *) ctx->h_tpw.p, *hm = hw + sel_bytes;
+
+    if (sel_off)
+    {
+        uint64_t *hs = (uint64_t *) hw;
+
+        for (size_t i = 0; i <= cnt; i++)
+            hs[i] = sel_off[lo + i] - sel_off[lo];
+        memcpy(hw + tp_al((cnt + 1) * 8), sel_pos + sel_off[lo], m * 4);
+        d_sel_off = (tup_u64 *) ((uint8_t *) work + work_bytes);
+        d_sel_pos = (uint32_t *) ((uint8_t *) d_sel_off + tp_al((cnt + 1) * 8));
+        CU(cudaMemcpyAsync(d_sel_off, hw, sel_bytes, cudaMemcpyHostToDevice, ctx->stream));
+        h2d += sel_bytes;
+    }
+    tup_u64 *d_bf = work + 3 * cnt + 1, *d_need = d_bf + cnt + 1;
+
+    rc = tuples_place(ctx->stream, cnt, d_blocks, stride, block_size, d_st, d_sel_off, d_sel_pos, ent_base, byte_base, data_cap,
+                      tup_cap, d_bf, d_st, d_need, work);
+    if (rc != CRYOGPU_OK)
+        return rc;
+    CU(cudaMemcpyAsync(hm, work + 2 * cnt, meta_words * 8, cudaMemcpyDeviceToHost, ctx->stream));
+    CU(cudaMemcpyAsync(hm + meta_words * 8, d_st, cnt * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    CU(cudaStreamSynchronize(ctx->stream));
+    d2h += meta_words * 8 + cnt * 4;
+    const uint64_t *h_byte_first = (const uint64_t *) hm, *h_bf = h_byte_first + cnt + 1, *h_need = h_bf + cnt + 1;
+    const int32_t  *h_st = (const int32_t *) (hm + meta_words * 8);
+    uint64_t        fit_e = 0, fit_b = 0;
+
+    /* the blocks that fit: one range of entries and bytes from ent_base / byte_base (once a block crosses a capacity,
+     * every later block with entries does) */
+    for (size_t i = 0; i < cnt; i++)
+        if (h_st[i] == CRYOGPU_ST_OK && h_bf[i + 1] > h_bf[i])
+        {
+            fit_e = h_bf[i + 1] - ent_base;
+            fit_b = h_byte_first[i + 1] - byte_base;
+        }
+    if (fit_e)
+    {
+        const size_t db = tp_al(fit_b), ob = tp_al(fit_e * 8), total = db + ob + fit_e * 4;
+        const bool   direct = is_pinned(data) && is_pinned(tup_off) && is_pinned(tup_len);
+
+        if ((rc = dev_reserve(ctx->tpo, total)) != CRYOGPU_OK || (!direct && (rc = host_reserve(ctx->h_tpo, total)) != CRYOGPU_OK))
+            return rc;
+        uint8_t     *o = (uint8_t *) ctx->tpo.p;
+        const TupOut to = {o, (tup_u64 *) (o + db), (uint32_t *) (o + db + ob), ent_base, byte_base};
+
+        if ((rc = tuples_gather(ctx->stream, cnt, d_blocks, stride, block_size, d_st, d_sel_off, d_sel_pos, d_bf, work, to)) !=
+            CRYOGPU_OK)
+            return rc;
+        if (direct)
+        {
+            CU(cudaMemcpyAsync((uint8_t *) data + byte_base, o, fit_b, cudaMemcpyDeviceToHost, ctx->stream));
+            CU(cudaMemcpyAsync(tup_off + ent_base, o + db, fit_e * 8, cudaMemcpyDeviceToHost, ctx->stream));
+            CU(cudaMemcpyAsync(tup_len + ent_base, o + db + ob, fit_e * 4, cudaMemcpyDeviceToHost, ctx->stream));
+            CU(cudaStreamSynchronize(ctx->stream));
+        }
+        else
+        {
+            uint8_t *h = (uint8_t *) ctx->h_tpo.p;
+
+            CU(cudaMemcpyAsync(h, o, fit_b, cudaMemcpyDeviceToHost, ctx->stream));
+            CU(cudaMemcpyAsync(h + db, o + db, ob + fit_e * 4, cudaMemcpyDeviceToHost, ctx->stream));
+            CU(cudaStreamSynchronize(ctx->stream));
+            memcpy((uint8_t *) data + byte_base, h, fit_b);
+            memcpy(tup_off + ent_base, h + db, fit_e * 8);
+            memcpy(tup_len + ent_base, h + db + ob, fit_e * 4);
+        }
+        d2h += fit_b + fit_e * 12;
+    }
+    CU(cudaEventRecord(ctx->busy, ctx->stream));
+    memcpy(status + lo, h_st, cnt * 4);
+    memcpy(block_first + lo, h_bf, cnt * 8);
+    ent_base += h_need[1];
+    byte_base += h_need[0];
+    return CRYOGPU_OK;
+}
+
+static int
+check_tuples_host_args(const cryogpu_ctx *ctx, uint32_t block_size, const uint64_t *sel_off, const uint32_t *sel_pos,
+                       const void *data, uint64_t data_cap, const uint64_t *tup_off, const uint32_t *tup_len, uint64_t tup_cap,
+                       const uint64_t *block_first, const int32_t *status, const uint64_t *need)
+{
+    if (!ctx)
+        return fail(CRYOGPU_E_ARG, "ctx is NULL");
+    if (!block_first || !status || !need || (sel_off && !sel_pos) || (data_cap && !data) || (tup_cap && (!tup_off || !tup_len)))
+        return fail(CRYOGPU_E_ARG, "NULL argument");
+    if (block_size < 16 || block_size > (1u << 27))
+        return fail(CRYOGPU_E_ARG, "block_size out of range");
+    return CRYOGPU_OK;
+}
+
+#define TUP_HOST_CHUNK 256u
+
+extern "C" int
+cryogpu_decompress_tuples_host(cryogpu_ctx *ctx, size_t n, const int32_t *methods, const void *const *src,
+                               const uint32_t *src_size, uint32_t block_size, const uint64_t *sel_off, const uint32_t *sel_pos,
+                               void *data, uint64_t data_cap, uint64_t *tup_off, uint32_t *tup_len, uint64_t tup_cap,
+                               uint64_t *block_first, int32_t *status, uint64_t *need)
+{
+    int rc = check_tuples_host_args(ctx, block_size, sel_off, sel_pos, data, data_cap, tup_off, tup_len, tup_cap, block_first,
+                                    status, need);
+
+    if (rc != CRYOGPU_OK)
+        return rc;
+    if (n && (!methods || !src || !src_size))
+        return fail(CRYOGPU_E_ARG, "NULL argument");
+    const uint64_t stride = ((uint64_t) block_size + 15) & ~(uint64_t) 15;
+    uint64_t       h2d = 0, d2h = 0, ent = 0, bytes = 0;
+    std::lock_guard<std::recursive_mutex> hold(ctx->mu);
+
+    CU(cudaSetDevice(ctx->device));
+    for (size_t lo = 0; lo < n; lo += TUP_HOST_CHUNK)
+    {
+        const size_t cnt = std::min<size_t>(TUP_HOST_CHUNK, n - lo);
+        size_t       in_bytes = 0;
+
+        for (size_t i = 0; i < cnt; i++)
+            in_bytes += ((size_t) src_size[lo + i] + 15) & ~(size_t) 15;
+        /* staging in: streams | offsets u64 | sizes u32 | methods i32 ; device out: blocks | out_size u32 | status i32 */
+        const size_t in_al = tp_al(in_bytes), meta_in = cnt * 16;
+
+        if ((rc = host_reserve(ctx->h_in[0], in_al + meta_in + 16)) != CRYOGPU_OK ||
+            (rc = dev_reserve(ctx->d_in[0], in_al + meta_in + 16)) != CRYOGPU_OK ||
+            (rc = dev_reserve(ctx->d_out[0], cnt * stride + cnt * 8)) != CRYOGPU_OK)
+            return rc;
+        uint8_t  *hi = (uint8_t *) ctx->h_in[0].p, *di = (uint8_t *) ctx->d_in[0].p, *dout = (uint8_t *) ctx->d_out[0].p;
+        uint64_t *h_off = (uint64_t *) (hi + in_al);
+        uint32_t *h_sz = (uint32_t *) (hi + in_al + cnt * 8);
+        int32_t  *h_me = (int32_t *) (hi + in_al + cnt * 12);
+        size_t    at = 0;
+
+        for (size_t i = 0; i < cnt; i++)
+        {
+            memcpy(hi + at, src[lo + i], src_size[lo + i]);
+            h_off[i] = at;
+            h_sz[i] = src_size[lo + i];
+            h_me[i] = methods[lo + i];
+            at += ((size_t) src_size[lo + i] + 15) & ~(size_t) 15;
+        }
+        CU(cudaMemcpyAsync(di, hi, in_al + meta_in, cudaMemcpyHostToDevice, ctx->stream));
+        h2d += in_al + meta_in;
+        uint32_t *d_osz = (uint32_t *) (dout + cnt * stride);
+        int32_t  *d_st = (int32_t *) (dout + cnt * stride + cnt * 4);
+
+        CU(cudaStreamWaitEvent(ctx->stream, ctx->busy, 0));
+        rc = decompress_device_locked(ctx, ctx->stream, cnt, (int32_t *) (di + in_al + cnt * 12), di, (uint64_t *) (di + in_al),
+                                      (uint32_t *) (di + in_al + cnt * 8), dout, stride, block_size, d_osz, d_st);
+        if (rc != CRYOGPU_OK)
+            return rc;
+        rc = tuples_chunk_host(ctx, lo, cnt, dout, stride, block_size, d_st, sel_off, sel_pos, data, data_cap, tup_off, tup_len,
+                               tup_cap, block_first, status, ent, bytes, h2d, d2h);
+        if (rc != CRYOGPU_OK)
+            return rc;
+    }
+    block_first[n] = ent;
+    need[0] = bytes;
+    need[1] = ent;
+    ctx->last_h2d = h2d;
+    ctx->last_d2h = d2h;
+    return CRYOGPU_OK;
+}
+
+extern "C" int
+cryogpu_decompress_pages_tuples_host(cryogpu_ctx *ctx, size_t n, const void *const *pages, const uint32_t *page_blkno,
+                                     const uint32_t *chain_off, uint32_t block_size, const uint64_t *sel_off,
+                                     const uint32_t *sel_pos, void *data, uint64_t data_cap, uint64_t *tup_off,
+                                     uint32_t *tup_len, uint64_t tup_cap, uint64_t *block_first, int32_t *status,
+                                     int32_t *methods, uint32_t *comp_size, uint64_t *need)
+{
+    int rc = check_tuples_host_args(ctx, block_size, sel_off, sel_pos, data, data_cap, tup_off, tup_len, tup_cap, block_first,
+                                    status, need);
+
+    if (rc != CRYOGPU_OK)
+        return rc;
+    if (n && (!pages || !page_blkno || !chain_off || !methods))
+        return fail(CRYOGPU_E_ARG, "NULL argument");
+    const uint64_t stride = ((uint64_t) block_size + 15) & ~(uint64_t) 15;
+    uint64_t       h2d = 0, d2h = 0, ent = 0, bytes = 0;
+    std::lock_guard<std::recursive_mutex> hold(ctx->mu);
+
+    CU(cudaSetDevice(ctx->device));
+    for (size_t lo = 0; lo < n; lo += PG_HOST_CHUNK)
+    {
+        const size_t   cnt = std::min<size_t>(PG_HOST_CHUNK, n - lo);
+        const uint32_t e0 = chain_off[lo], e1 = chain_off[lo + cnt], ne = e1 - e0;
+
+        if (e1 < e0)
+            return fail(CRYOGPU_E_ARG, "chain_off must not decrease");
+        if (ne == 0)
+        {
+            for (size_t i = 0; i < cnt; i++)
+            {
+                status[lo + i] = CRYOGPU_ST_EMPTY_BLOCK;
+                block_first[lo + i] = ent;
+                methods[lo + i] = 0;
+                if (comp_size)
+                    comp_size[lo + i] = 0;
+            }
+            continue;
+        }
+        /* staging in: pages | slot | blkno | chain_off (cnt + 1); device out: blocks | out_size | status | methods | comp_size */
+        const size_t pg_bytes = (size_t) ne * PG_PAGE, meta_in = tp_al((size_t) ne * 8 + (cnt + 1) * 4);
+
+        if ((rc = host_reserve(ctx->h_in[0], pg_bytes + meta_in)) != CRYOGPU_OK ||
+            (rc = dev_reserve(ctx->d_in[0], pg_bytes + meta_in)) != CRYOGPU_OK ||
+            (rc = host_reserve(ctx->h_out[0], cnt * 8)) != CRYOGPU_OK ||
+            (rc = dev_reserve(ctx->d_out[0], cnt * stride + cnt * 16)) != CRYOGPU_OK)
+            return rc;
+        uint8_t  *hi = (uint8_t *) ctx->h_in[0].p, *di = (uint8_t *) ctx->d_in[0].p, *dout = (uint8_t *) ctx->d_out[0].p;
+        uint32_t *h_slot = (uint32_t *) (hi + pg_bytes), *h_blk = h_slot + ne, *h_coff = h_blk + ne;
+
+        host_pool(ctx)->run((ne + 255) / 256, [&](size_t part) {
+            for (uint32_t e = (uint32_t) part * 256u; e < ne && e < (uint32_t) (part + 1) * 256u; e++)
+            {
+                memcpy(hi + (size_t) e * PG_PAGE, pages[e0 + e], PG_PAGE);
+                h_slot[e] = e;
+                h_blk[e] = page_blkno[e0 + e];
+            }
+        });
+        for (size_t i = 0; i <= cnt; i++)
+            h_coff[i] = chain_off[lo + i] - e0;
+        CU(cudaMemcpyAsync(di, hi, pg_bytes + meta_in, cudaMemcpyHostToDevice, ctx->stream));
+        h2d += pg_bytes + meta_in;
+        uint8_t *dm = dout + cnt * stride;
+        int32_t *d_st = (int32_t *) (dm + cnt * 4);
+
+        rc = cryogpu_decompress_pages_device(ctx, cnt, di, (uint32_t *) (di + pg_bytes), (uint32_t *) (di + pg_bytes) + ne,
+                                             (uint32_t *) (di + pg_bytes) + 2 * (size_t) ne, ne, dout, stride, block_size,
+                                             (uint32_t *) dm, d_st, (int32_t *) (dm + cnt * 8), (uint32_t *) (dm + cnt * 12),
+                                             ctx->stream);
+        if (rc != CRYOGPU_OK)
+            return rc;
+        /* methods | comp_size: read once the chunk's tuples are back (tuples_chunk_host waits for the stream) */
+        CU(cudaMemcpyAsync(ctx->h_out[0].p, dm + cnt * 8, cnt * 8, cudaMemcpyDeviceToHost, ctx->stream));
+        d2h += cnt * 8;
+        rc = tuples_chunk_host(ctx, lo, cnt, dout, stride, block_size, d_st, sel_off, sel_pos, data, data_cap, tup_off, tup_len,
+                               tup_cap, block_first, status, ent, bytes, h2d, d2h);
+        if (rc != CRYOGPU_OK)
+            return rc;
+        memcpy(methods + lo, ctx->h_out[0].p, cnt * 4);
+        if (comp_size)
+            memcpy(comp_size + lo, (const uint8_t *) ctx->h_out[0].p + cnt * 4, cnt * 4);
+    }
+    block_first[n] = ent;
+    need[0] = bytes;
+    need[1] = ent;
     ctx->last_h2d = h2d;
     ctx->last_d2h = d2h;
     return CRYOGPU_OK;

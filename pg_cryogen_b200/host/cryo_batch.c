@@ -22,6 +22,36 @@ static uint32_t rd16(const uint8_t *p) { uint16_t v; memcpy(&v, p, 2); return v;
 
 /* ------------------------------------------------------------------ read side */
 
+/*
+ * The pages of the chain that starts at blk, following `next` as cache.c:151-176 does: the device needs the pages, the
+ * host finds them.  An empty or foreign first page still goes to the device alone: it names the error (cache.c:112-129).
+ * Fills pages[] / pblk[] (CRYO_BATCH_MAXPAGES at most) and returns their number; *xid: created_xid of a first page.
+ */
+static uint32_t
+walk_chain(const CryoRelOps *ops, uint32_t blk, uint32_t relblocks, const void **pages, uint32_t *pblk, uint32_t *xid)
+{
+    const uint8_t *pg = ops->read_page(ops->rel, blk);
+    uint32_t       want = 0, k = 0;
+
+    if (pg && rd16(pg + OFF_PD_UPPER) != 0 && rd32(pg + OFF_FIRST) == blk)
+    {
+        want = rd16(pg + OFF_NPAGES);
+        *xid = rd32(pg + OFF_XID);
+    }
+    while (pg && k < CRYO_BATCH_MAXPAGES)
+    {
+        pages[k] = pg;
+        pblk[k++] = blk;
+        if (k >= want)
+            break;
+        blk = rd32(pg + OFF_NEXT);
+        if (blk == INVALID_BLOCK || blk >= relblocks)
+            break;
+        pg = ops->read_page(ops->rel, blk);
+    }
+    return k;
+}
+
 typedef struct
 {
     uint32_t    blockno;        /* key (one relation per cache here; the reference keys by (relid, blockno)) */
@@ -168,32 +198,14 @@ cryo_batch_read_data(CryoBatchCache *c, const CryoRelOps *ops, const uint32_t *b
             rc = CRYOGPU_E_NOMEM;
             goto done;
         }
-        /* walk `next` from each first page, as cache.c:151-176 does: the device needs the pages, the host finds them */
         for (int m = 0; m < nmiss; m++)
         {
-            Slot          *s = &c->slot[entries[miss[m]]];
-            uint32_t       blk = s->blockno, want = 0;
-            const uint8_t *pg = ops->read_page(ops->rel, blk);
+            Slot *s = &c->slot[entries[miss[m]]];
 
             coff[m] = (uint32_t) npages;
-            if (pg && rd16(pg + OFF_PD_UPPER) != 0 && rd32(pg + OFF_FIRST) == blk)
-            {
-                want = rd16(pg + OFF_NPAGES);
-                s->xid = rd32(pg + OFF_XID);
-            }
-            /* an empty or foreign first page still goes to the device: it names the error (cache.c:112-129) */
-            while (pg && s->nblocks < CRYO_BATCH_MAXPAGES)
-            {
-                pages[npages] = pg;
-                pblk[npages++] = blk;
-                s->blocks[s->nblocks++] = blk;
-                if (s->nblocks >= want)
-                    break;
-                blk = rd32(pg + OFF_NEXT);
-                if (blk == INVALID_BLOCK || blk >= relblocks)
-                    break;
-                pg = ops->read_page(ops->rel, blk);
-            }
+            s->nblocks = walk_chain(ops, s->blockno, relblocks, pages + npages, pblk + npages, &s->xid);
+            memcpy(s->blocks, pblk + npages, sizeof(uint32_t) * s->nblocks);
+            npages += s->nblocks;
         }
         coff[nmiss] = (uint32_t) npages;
         void    **dst = malloc(sizeof(void *) * (size_t) nmiss);
@@ -369,6 +381,196 @@ cryo_batch_scan_end(CryoBatchScan *s)
     free(s->win_entry);
     free(s->win_err);
     free(s);
+}
+
+/* ---- TID fetch ---- */
+
+static int
+cmp_u64(const void *a, const void *b)
+{
+    const uint64_t x = *(const uint64_t *) a, y = *(const uint64_t *) b;
+
+    return x < y ? -1 : x > y;
+}
+
+static CryoError
+fetch_error(int32_t st)
+{
+    return st == CRYOGPU_ST_OK ? CRYO_ERR_SUCCESS
+           : st == CRYOGPU_ST_EMPTY_BLOCK ? CRYO_ERR_EMPTY_BLOCK
+           : st == CRYOGPU_ST_WRONG_START ? CRYO_ERR_WRONG_STARTING_BLOCK
+           : CRYO_ERR_DECOMPRESSION_FAILED;
+}
+
+#define FETCH_GUESS_TUPLE   8192u       /* output room guessed per single position: a heap page */
+#define FETCH_GUESS_ITEMS   290u        /* entries guessed per position 0: storage.c's limit per block */
+
+int
+cryo_batch_fetch_tuples(cryogpu_ctx *gpu, const CryoRelOps *ops, const uint32_t *tid_block, const uint32_t *tid_pos, int m,
+                        CryoFetchResult *res)
+{
+    const uint32_t relblocks = ops->nblocks(ops->rel);
+    uint64_t   *key = malloc(sizeof(uint64_t) * (size_t) (m > 0 ? m : 1));
+    int         nk = 0, nb = 0, rc = 0;
+    uint32_t   *blk = NULL, *pblk = NULL, *coff = NULL, *sel_pos = NULL, *bxid = NULL;
+    uint64_t   *sel_off = NULL, *bf = NULL, *rfirst = NULL, *rcount = NULL, dcap = 0, tcap = 0, need[2] = {0, 0};
+    int32_t    *st = NULL, *me = NULL;
+    const void **pages = NULL;
+    size_t      npages = 0;
+
+    memset(res, 0, sizeof(*res));
+    res->err = calloc((size_t) (m > 0 ? m : 1), sizeof(CryoError));
+    res->xid = calloc((size_t) (m > 0 ? m : 1), sizeof(uint32_t));
+    res->first = calloc((size_t) m + 1, sizeof(uint64_t));
+    rfirst = calloc((size_t) (m > 0 ? m : 1), sizeof(uint64_t));
+    rcount = calloc((size_t) (m > 0 ? m : 1), sizeof(uint64_t));
+    if (!key || !res->err || !res->xid || !res->first || !rfirst || !rcount)
+    {
+        rc = CRYOGPU_E_NOMEM;
+        goto done;
+    }
+    /* cache.c:256-260: the metapage and blocks past the end; the others grouped by block, in request order */
+    for (int i = 0; i < m; i++)
+        if (tid_block[i] >= relblocks || tid_block[i] == 0)
+            res->err[i] = CRYO_ERR_WRONG_STARTING_BLOCK;
+        else
+            key[nk++] = (uint64_t) tid_block[i] << 32 | (uint32_t) i;
+    qsort(key, (size_t) nk, sizeof(uint64_t), cmp_u64);
+    for (int k = 0; k < nk; k++)
+        nb += k == 0 || (key[k] >> 32) != (key[k - 1] >> 32);
+    blk = malloc(sizeof(uint32_t) * (size_t) (nb + 1));
+    bxid = calloc((size_t) nb + 1, sizeof(uint32_t));
+    coff = malloc(sizeof(uint32_t) * (size_t) (nb + 1));
+    sel_off = malloc(sizeof(uint64_t) * (size_t) (nb + 1));
+    bf = malloc(sizeof(uint64_t) * (size_t) (nb + 1));
+    sel_pos = malloc(sizeof(uint32_t) * (size_t) (nk + 1));
+    st = malloc(sizeof(int32_t) * (size_t) (nb + 1));
+    me = malloc(sizeof(int32_t) * (size_t) (nb + 1));
+    pages = malloc(sizeof(void *) * (size_t) (nb + 1) * CRYO_BATCH_MAXPAGES);
+    pblk = malloc(sizeof(uint32_t) * (size_t) (nb + 1) * CRYO_BATCH_MAXPAGES);
+    if (!blk || !bxid || !coff || !sel_off || !bf || !sel_pos || !st || !me || !pages || !pblk)
+    {
+        rc = CRYOGPU_E_NOMEM;
+        goto done;
+    }
+    /* one walk per distinct block; its positions in request order (repeats and all) */
+    nb = 0;
+    for (int k = 0; k < nk; k++)
+    {
+        const uint32_t b = (uint32_t) (key[k] >> 32), pos = tid_pos[(uint32_t) key[k]];
+
+        if (k == 0 || b != blk[nb - 1])
+        {
+            blk[nb] = b;
+            sel_off[nb] = (uint64_t) k;
+            coff[nb] = (uint32_t) npages;
+            npages += walk_chain(ops, b, relblocks, pages + npages, pblk + npages, &bxid[nb]);
+            nb++;
+        }
+        sel_pos[k] = pos;
+        tcap += pos ? 1u : FETCH_GUESS_ITEMS;
+        dcap += pos ? FETCH_GUESS_TUPLE : CRYO_BATCH_BLCKSZ;
+    }
+    sel_off[nb] = (uint64_t) nk;
+    coff[nb] = (uint32_t) npages;
+    /* one device call; a second one only when the guessed room was short (need says how much there is to fetch) */
+    for (int attempt = 0; nb && attempt < 2; attempt++)
+    {
+        free(res->data_);
+        free(res->tup_off_);
+        free(res->tup_len_);
+        res->data_ = malloc(dcap ? dcap : 1);
+        res->tup_off_ = malloc(sizeof(uint64_t) * (tcap ? tcap : 1));
+        res->tup_len_ = malloc(sizeof(uint32_t) * (tcap ? tcap : 1));
+        if (!res->data_ || !res->tup_off_ || !res->tup_len_)
+        {
+            rc = CRYOGPU_E_NOMEM;
+            goto done;
+        }
+        rc = cryogpu_decompress_pages_tuples_host(gpu, (size_t) nb, pages, pblk, coff, CRYO_BATCH_BLCKSZ, sel_off, sel_pos,
+                                                  res->data_, dcap, res->tup_off_, res->tup_len_, tcap, bf, st, me, NULL, need);
+        res->calls++;
+        if (rc != 0 || (need[0] <= dcap && need[1] <= tcap))
+            break;
+        dcap = need[0];
+        tcap = need[1];
+    }
+    if (rc != 0)
+        goto done;
+    /* per request: its block's error and xid, and its entries (a position 0 has the block's ntuples of them) */
+    for (int d = 0, k = 0; d < nb; d++)
+    {
+        const CryoError e = fetch_error(st[d]);
+        uint64_t        zeros = 0, ent = bf[d];
+
+        for (uint64_t s = sel_off[d]; s < sel_off[d + 1]; s++)
+            zeros += sel_pos[s] == 0;
+        const uint64_t nt = zeros ? (bf[d + 1] - bf[d] - (sel_off[d + 1] - sel_off[d] - zeros)) / zeros : 0;
+
+        for (; k < nk && (uint32_t) (key[k] >> 32) == blk[d]; k++)
+        {
+            const uint32_t i = (uint32_t) key[k];
+
+            res->err[i] = e;
+            if (e != CRYO_ERR_SUCCESS)
+                continue;
+            res->xid[i] = bxid[d];
+            rfirst[i] = ent;
+            rcount[i] = sel_pos[k] ? 1u : nt;
+            ent += rcount[i];
+        }
+    }
+    for (int i = 0; i < m; i++)
+        res->first[i + 1] = res->first[i] + rcount[i];
+    res->ntuples = res->first[m];
+    res->tuple = malloc(sizeof(char *) * (size_t) (res->ntuples ? res->ntuples : 1));
+    res->len = malloc(sizeof(uint32_t) * (size_t) (res->ntuples ? res->ntuples : 1));
+    if (!res->tuple || !res->len)
+    {
+        rc = CRYOGPU_E_NOMEM;
+        goto done;
+    }
+    for (int i = 0; i < m; i++)
+        for (uint64_t j = 0; j < rcount[i]; j++)
+        {
+            const uint64_t e = rfirst[i] + j, t = res->first[i] + j;
+
+            res->tuple[t] = res->tup_off_[e] == UINT64_MAX ? NULL : (const char *) res->data_ + res->tup_off_[e];
+            res->len[t] = res->tup_len_[e];
+        }
+done:
+    if (rc != 0)
+        for (int i = 0; i < m; i++)
+            if (res->err)
+                res->err[i] = CRYO_ERR_DECOMPRESSION_FAILED;
+    free(key);
+    free(blk);
+    free(bxid);
+    free(coff);
+    free(sel_off);
+    free(bf);
+    free(sel_pos);
+    free(st);
+    free(me);
+    free(pages);
+    free(pblk);
+    free(rfirst);
+    free(rcount);
+    return rc;
+}
+
+void
+cryo_fetch_result_free(CryoFetchResult *res)
+{
+    free(res->err);
+    free(res->xid);
+    free(res->first);
+    free(res->tuple);
+    free(res->len);
+    free(res->data_);
+    free(res->tup_off_);
+    free(res->tup_len_);
+    memset(res, 0, sizeof(*res));
 }
 
 /* ----------------------------------------------------------------- write side */

@@ -81,6 +81,30 @@ CryoBatchScan *cryo_batch_scan_begin(CryoBatchCache *c, const CryoRelOps *ops, i
 char       *cryo_batch_scan_next(CryoBatchScan *s, uint32_t *blockno, uint32_t *xid, CryoError *err);
 void        cryo_batch_scan_end(CryoBatchScan *s);
 
+/* TID fetch: the random-read path (index fetch, bitmap heap scan, row lock, analyze; cryo_read_data + cryo_storage_fetch,
+ * pg_cryogen.c:377-463, :862-895, :987-1034) for m TIDs at once.  Each distinct block's chain is walked once on the host
+ * and all of them go to ONE cryogpu_decompress_pages_tuples_host call (a second one only when the tuples outgrow the
+ * room guessed for them); only the selected tuples come back.  Not through the block cache. */
+typedef struct
+{
+    CryoError  *err;            /* [m]: what cryo_read_data returns for the request's block */
+    uint32_t   *xid;            /* [m]: the block's created_xid, for the visibility rule of pg_cryogen.c:282-290 */
+    uint64_t   *first;          /* [m + 1]: request i's tuples are [first[i], first[i + 1]): one, or every item for 0 */
+    const char **tuple;         /* the tuple's bytes (MAXALIGNed), NULL when the position does not exist */
+    uint32_t   *len;
+    uint64_t    ntuples;
+    uint64_t    calls;          /* device calls made */
+    void       *data_;          /* private: the packed tuples and their entries */
+    uint64_t   *tup_off_;
+    uint32_t   *tup_len_;
+} CryoFetchResult;
+
+/* tid_block[i], tid_pos[i]: ItemPointer i (the block of the cryo block's first page, a 1-based item position; 0 = every
+ * item of the block, as a lossy bitmap page asks).  Returns 0 or a cryogpu call code; free the result either way. */
+int         cryo_batch_fetch_tuples(cryogpu_ctx *gpu, const CryoRelOps *ops, const uint32_t *tid_block, const uint32_t *tid_pos,
+                                    int m, CryoFetchResult *res);
+void        cryo_fetch_result_free(CryoFetchResult *res);
+
 /* write side */
 typedef struct CryoBatchWriter CryoBatchWriter;
 CryoBatchWriter *cryo_batch_writer_create(cryogpu_ctx *gpu, const CryoRelOps *ops, int method, int level_or_accel,
