@@ -262,6 +262,41 @@ int cryogpu_compress_pages_alloc_host(cryogpu_ctx *ctx, size_t n, int method, in
                                       uint32_t *npages, uint32_t *comp_size, int32_t *status);
 
 /*
+ * ------------------------------------------------------------ cryo blocks from packed tuples
+ *
+ * The write-side mirror of the batched tuple fetch below: tuples in the layout it returns -- entry e is
+ * (tup_off[e], tup_len[e]) into data, block i takes entries [block_first[i], block_first[i + 1]) in insertion
+ * order -- and block i out as cryo_init_page + cryo_storage_insert (storage.c:15-50) build it, byte for byte:
+ * header {lower, upper}, item j {off, len} at byte 8 + 8j, tuple j at block_size - sum over k <= j of
+ * MAXALIGN(len_k), every other byte zero.  block_size must be a multiple of 8 (else CRYOGPU_E_ARG).
+ *
+ *   status[i]   CRYOGPU_ST_FORMAT: block_first[i + 1] < block_first[i], or an entry with tup_off == UINT64_MAX (the
+ *               fetch's "not found"), len > block_size, or bytes outside [0, data_size).  CRYOGPU_ST_OUTPUT:
+ *               storage_insert would not take every entry (more than 290 items, or a tuple that does not fit).
+ *               A failed block is not written.
+ *
+ * Bytes: read sum len + 12 per entry; write n * block_size.
+ */
+
+/* Blocks from tuples, everything in HBM (d_data any alignment; d_dst, dst_stride multiples of 16).  Enqueues work on
+ * `stream` only; calls on one context are ordered as the other device-resident calls are. */
+int cryogpu_build_blocks_device(cryogpu_ctx *ctx, size_t n, const uint8_t *d_data, uint64_t data_size,
+                                const uint64_t *d_tup_off, const uint32_t *d_tup_len, const uint64_t *d_block_first,
+                                uint32_t block_size, uint8_t *d_dst, uint64_t dst_stride, int32_t *d_status,
+                                void *stream);
+
+/* The COPY flush from tuples: as cryogpu_compress_pages_alloc_host, but the blocks are built on the device, so only
+ * the entries and the bytes of data they cover cross the bus (straight from pinned memory where the caller's is).
+ * A block whose build failed has that status, asks alloc for no page and writes nothing.  block_first must not
+ * decrease (else CRYOGPU_E_ARG).  cryogpu_last_transfer_bytes reports the bytes moved. */
+int cryogpu_compress_tuples_pages_alloc_host(cryogpu_ctx *ctx, size_t n, int method, int level_or_accel,
+                                             const void *data, uint64_t data_size, const uint64_t *tup_off,
+                                             const uint32_t *tup_len, const uint64_t *block_first, uint32_t block_size,
+                                             const uint32_t *first_blkno, cryogpu_alloc_page_fn alloc,
+                                             cryogpu_page_ptr_fn page_ptr, void *arg, uint32_t created_xid,
+                                             uint32_t *npages, uint32_t *comp_size, int32_t *status);
+
+/*
  * ------------------------------------------------------------ tuple-level work
  *
  * The item walk of a sequential scan (cryo_getnextslot, pg_cryogen.c:293-307, over cryo_storage_fetch,

@@ -74,6 +74,12 @@ _PROTOS = {
     "cryogpu_compress_pages_alloc_host": (C.c_int, [C.c_void_p, C.c_size_t, C.c_int, C.c_int, C.c_void_p, C.c_uint32,
                                                     C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32,
                                                     C.c_void_p, C.c_void_p, C.c_void_p]),
+    "cryogpu_build_blocks_device": (C.c_int, [C.c_void_p, C.c_size_t, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p,
+                                              C.c_void_p, C.c_uint32, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p]),
+    "cryogpu_compress_tuples_pages_alloc_host": (C.c_int, [C.c_void_p, C.c_size_t, C.c_int, C.c_int, C.c_void_p, C.c_uint64,
+                                                           C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p,
+                                                           C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p,
+                                                           C.c_void_p, C.c_void_p]),
     "cryogpu_tuple_stats_device": (C.c_int, [C.c_void_p, C.c_size_t, C.c_void_p, C.c_uint64, C.c_uint32, C.c_void_p,
                                              C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "cryogpu_decompress_count_host": (C.c_int, [C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32,
@@ -364,6 +370,56 @@ class CryoGPU:
                                                                  block_size, so, sp, data, dcap, to, tl, tcap, bf, st,
                                                                  me.ctypes.data, csz.ctypes.data, need)
         return self._tuples_host(call, "cryogpu_decompress_pages_tuples_host", n, sel, data_cap, tup_cap) + (me, csz)
+
+    # ---- cryo blocks from packed tuples (the write-side mirror of the tuple fetch) ----
+
+    def build_blocks_device(self, data, data_size: int, tup_off, tup_len, block_first, n: int, dst, dst_stride: int, status,
+                            block_size: int = CRYO_BLCKSZ, stream: int | None = None):
+        """Packed tuples in HBM -> cryo blocks at dst + i * dst_stride (torch CUDA tensors or device pointers); only
+        enqueues."""
+        self._check(self.lib.cryogpu_build_blocks_device(
+            self.handle, n, _ptr(data), data_size, _ptr(tup_off), _ptr(tup_len), _ptr(block_first), block_size, _ptr(dst),
+            dst_stride, _ptr(status), _stream(stream)), "cryogpu_build_blocks_device")
+
+    def compress_tuples_pages_host(self, method: int, level_or_accel: int, data: np.ndarray, tup_off: np.ndarray,
+                                   tup_len: np.ndarray, block_first: np.ndarray, relation: np.ndarray, first_blkno,
+                                   next_blkno: int, created_xid: int, block_size: int = CRYO_BLCKSZ):
+        """The COPY flush from packed tuples into relation [npages, 8192] (indexed by block number): block i's first
+        page is first_blkno[i], further pages are handed out from next_blkno on.  Returns (npages, comp_size, status,
+        the block numbers handed out in order)."""
+        n = block_first.size - 1
+        data = np.ascontiguousarray(data, dtype=np.uint8)
+        to = np.ascontiguousarray(tup_off, dtype=np.uint64)
+        tl = np.ascontiguousarray(tup_len, dtype=np.uint32)
+        bf = np.ascontiguousarray(block_first, dtype=np.uint64)
+        first = np.ascontiguousarray(first_blkno, dtype=np.uint32)
+        alloc, page_ptr, handed = page_callbacks(relation, next_blkno)
+        npg = np.zeros(max(n, 1), dtype=np.uint32)
+        csz = np.zeros(max(n, 1), dtype=np.uint32)
+        st = np.full(max(n, 1), -1, dtype=np.int32)
+        self._check(self.lib.cryogpu_compress_tuples_pages_alloc_host(
+            self.handle, n, method, level_or_accel, data.ctypes.data, data.size, to.ctypes.data, tl.ctypes.data,
+            bf.ctypes.data, block_size, first.ctypes.data, alloc, page_ptr, None, created_xid, npg.ctypes.data,
+            csz.ctypes.data, st.ctypes.data), "cryogpu_compress_tuples_pages_alloc_host")
+        return npg[:n], csz[:n], st[:n], handed
+
+
+ALLOC_PAGE_FN = C.CFUNCTYPE(C.c_uint32, C.c_void_p)
+PAGE_PTR_FN = C.CFUNCTYPE(C.c_void_p, C.c_void_p, C.c_uint32)
+
+
+def page_callbacks(relation: np.ndarray, next_blkno: int):
+    """(alloc, page_ptr, handed) for the *_pages_alloc_host calls over relation [npages, 8192]: alloc hands out
+    next_blkno, next_blkno + 1, ... and records them in the list `handed`; page_ptr(b) is relation[b]."""
+    handed = []
+
+    def alloc(_arg):
+        handed.append(next_blkno + len(handed))
+        return handed[-1]
+
+    def page_ptr(_arg, b):
+        return relation[b].ctypes.data if b < relation.shape[0] else None
+    return ALLOC_PAGE_FN(alloc), PAGE_PTR_FN(page_ptr), handed
 
 
 def _sel_arrays(sel, n: int):

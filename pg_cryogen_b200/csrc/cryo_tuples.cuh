@@ -18,6 +18,9 @@
  * Output: tuples start on 8-byte boundaries (a HeapTupleHeader pointer into the buffer is MAXALIGNed); the pad
  * bytes up to MAXALIGN(len) are zero.  A position outside 1..ntuples gives tup_off = TUP_NONE, tup_len = 0.
  * Blocks are 8-byte aligned (stride too); the data buffer is 16-byte aligned.
+ *
+ * The write side runs the other way (blk_build_block, the COPY flush from packed tuples): entries in the layout the
+ * gather writes in, cryo blocks out, byte for byte what cryo_init_page + cryo_storage_insert (storage.c:15-50) build.
  */
 #pragma once
 #include "cryo_common.cuh"
@@ -360,4 +363,129 @@ CRYO_DEV void tup_gather_block(const uint8_t *block, uint32_t block_size, const 
             cur = z + 1u;
         }
     }
+}
+
+/* ---------------------------------------------------------------- block build */
+
+#define BLK_THREADS     256u
+#define BLK_MAX_ITEMS   290u                    /* storage.c: (lower - 8) / 8 + 1 >= MaxHeapTuplesPerPage (291) rejects */
+#define BLK_SMEM        (BLK_MAX_ITEMS * 4u + 8u * 8u + 8u)     /* upper_j per entry | warp sums | two flags */
+
+static_assert(2u * BLK_THREADS >= BLK_MAX_ITEMS, "the scan gives each thread two entries");
+
+/*
+ * One cryo block from its entries [block_first[b], block_first[b + 1]) of (tup_off, tup_len), in insertion order,
+ * by one CTA of BLK_THREADS threads.  Tuple bytes are read at data + (tup_off - data_lo); an entry is malformed
+ * (CRYOGPU_ST_FORMAT) when tup_off is TUP_NONE, len > block_size, or [tup_off, tup_off + len) is not inside
+ * [data_lo, data_size).  A block storage.c would not take in full is CRYOGPU_ST_OUTPUT.  A failed block writes nothing.
+ *
+ * Acceptance is storage_insert's rule for every entry at once: with S_j = sum over k < j of MAXALIGN(len_k), before
+ * entry j lower = 8 + 8j and upper = block_size - S_j, and j is taken iff len_j + 8 <= upper - lower and j < 290.
+ *
+ * block_size % 8 == 0 (the caller checks) keeps every lower and upper a multiple of 8, so a taken entry has
+ * MAXALIGN(len_j) <= upper - lower - 8: its tuple [upper - MAXALIGN(len_j), upper) lies above its item
+ * [lower, lower + 8), and the final block splits into disjoint ranges -- header [0, 8), items [8, lower), the zero
+ * gap [lower, upper), tuples and their zero pad [upper, block_size).  The writes below rely on that: they go in any
+ * order, by any thread, with no barrier between them.
+ */
+CRYO_DEV void blk_build_block(const uint8_t *data, tup_u64 data_lo, tup_u64 data_size, const tup_u64 *tup_off,
+                              const uint32_t *tup_len, const tup_u64 *block_first, uint32_t b, uint32_t block_size,
+                              uint8_t *dst, int32_t *status, uint32_t *smem, uint32_t tid)
+{
+    uint32_t *s_up = smem, *s_flag = smem + BLK_MAX_ITEMS + 16u;
+    tup_u64  *s_warp = reinterpret_cast<tup_u64 *>(smem + BLK_MAX_ITEMS);
+    const uint32_t lane = tid & 31u, w = tid >> 5;
+    const tup_u64 e0 = block_first[b], e1 = block_first[b + 1];
+    const tup_u64 cnt = e1 >= e0 ? e1 - e0 : 0u;
+    bool bad = e1 < e0;
+
+    if (tid == 0)
+        s_flag[0] = s_flag[1] = 0u;
+    for (tup_u64 k = tid; k < cnt; k += BLK_THREADS)
+    {
+        const tup_u64 off = tup_off[e0 + k], len = tup_len[e0 + k];
+
+        if (off == TUP_NONE || len > block_size || off < data_lo || off > data_size || len > data_size - off)
+            bad = true;
+    }
+    __syncthreads();
+    if (bad)
+        s_flag[0] = 1u;
+    __syncthreads();
+    if (s_flag[0] || cnt > BLK_MAX_ITEMS)
+    {
+        if (tid == 0)
+            *status = s_flag[0] ? ST_FORMAT : ST_OUTPUT;
+        return;
+    }
+    /* exclusive prefix sums of MAXALIGN(len): thread t holds entries 2t and 2t + 1 */
+    const uint32_t j0 = 2u * tid, n = (uint32_t) cnt;
+    const uint32_t l0 = j0 < n ? tup_len[e0 + j0] : 0u, l1 = j0 + 1u < n ? tup_len[e0 + j0 + 1u] : 0u;
+    const tup_u64 a0 = tup_maxalign(l0), mine = a0 + tup_maxalign(l1);
+    tup_u64 x = mine;
+
+    for (uint32_t d = 1; d < 32u; d <<= 1)
+    {
+        const tup_u64 y = __shfl_up_sync(CRYO_FULL, x, d);
+
+        if (lane >= d)
+            x += y;
+    }
+    if (lane == 31u)
+        s_warp[w] = x;
+    __syncthreads();
+    tup_u64 s = x - mine;
+
+    for (uint32_t k = 0; k < w; k++)
+        s += s_warp[k];
+    /* entry j is taken iff len_j + 8 <= (block_size - S_j) - (8 + 8j); signed: past a refused entry it can go negative */
+    bool refuse = false;
+
+    for (uint32_t i = 0; i < 2u; i++)
+    {
+        const uint32_t j = j0 + i, len = i ? l1 : l0;
+
+        if (j >= n)
+            break;
+        const long long room = (long long) block_size - (long long) s - 8ll - 8ll * j;
+
+        if ((long long) len + 8ll > room)
+            refuse = true;
+        s += tup_maxalign(len);
+        s_up[j] = (uint32_t) (block_size - s);         /* upper_j, meaningful when every entry is taken */
+    }
+    if (refuse)
+        s_flag[1] = 1u;
+    __syncthreads();
+    if (s_flag[1])
+    {
+        if (tid == 0)
+            *status = ST_OUTPUT;
+        return;
+    }
+    const uint32_t lower = 8u + 8u * n, upper = n ? s_up[n - 1u] : block_size;
+
+    /* header, items */
+    if (tid == 0)
+    {
+        *status = ST_OK;
+        tup_st8(dst, (tup_u64) upper << 32 | lower);
+    }
+    for (uint32_t i = 0; i < 2u && j0 + i < n; i++)
+        tup_st8(dst + 8u + 8u * (j0 + i), (tup_u64) (i ? l1 : l0) << 32 | s_up[j0 + i]);
+    /* the zero gap [lower, upper): 16-byte stores over its aligned middle, one 8-byte word at either end at most */
+    {
+        const uint32_t a = (lower + 15u) & ~15u, z = upper & ~15u;
+
+        if (tid == 0 && lower < a && lower < upper)
+            tup_st8(dst + lower, 0ull);
+        if (tid == 1 && a <= upper && z < upper && z >= a)
+            tup_st8(dst + z, 0ull);
+        if (a < z)
+            for (uint32_t v = tid; v < (z - a) / 16u; v += BLK_THREADS)
+                st16(dst + a + 16u * v, make_uint4(0u, 0u, 0u, 0u));
+    }
+    /* tuples, zero-padded to MAXALIGN(len): one 8-lane group each (a team of 8 moves a 128-byte line per step) */
+    for (uint32_t j = tid >> 3; j < n; j += BLK_THREADS / 8u)
+        tup_copy(dst + s_up[j], data + (tup_off[e0 + j] - data_lo), tup_len[e0 + j], tid & 7u, 8u);
 }

@@ -900,6 +900,17 @@ k_tuple_gather(const uint8_t *blocks, uint64_t stride, uint32_t block_size, cons
         tup_gather_block(blocks + b * stride, block_size, sel_off, sel_pos, b, block_first[b], byte_first[b], o, lane);
 }
 
+/* cryo blocks from packed tuples (cryo_tuples.cuh): one CTA per block */
+__global__ void __launch_bounds__(BLK_THREADS)
+k_block_build(const uint8_t *data, tup_u64 data_lo, tup_u64 data_size, const tup_u64 *tup_off, const uint32_t *tup_len,
+              const tup_u64 *block_first, uint32_t block_size, uint8_t *dst, uint64_t dst_stride, int32_t *status)
+{
+    const uint32_t b = blockIdx.x;
+
+    blk_build_block(data, data_lo, data_size, tup_off, tup_len, block_first, b, block_size, dst + b * dst_stride, status + b,
+                    (uint32_t *) CRYO_SMEM_BASE(), threadIdx.x);
+}
+
 /* CRYOGPU_LZ4_KERNEL = warp | cx forces one LZ4 decoder for every block; default: routed per block */
 static int
 lz4_kernel_choice()
@@ -1941,6 +1952,7 @@ cryogpu_compress_device(cryogpu_ctx *ctx, size_t n, int method, int level_or_acc
 
 static HostPool *host_pool(cryogpu_ctx *ctx);
 static bool is_pinned(const void *p);
+static size_t tp_al(size_t v);
 
 extern "C" uint32_t
 cryogpu_pages_needed(uint64_t compressed_size)
@@ -2236,7 +2248,91 @@ cryogpu_compress_pages_host(cryogpu_ctx *ctx, size_t n, int method, int level_or
  * them then too: the first page was reserved when the block was started (cryo_reserve_blockno,
  * pg_cryogen.c:588-601), the others come from ReadBuffer(P_NEW) -- then cut the page images on the device
  * and place them where the caller says each page lives.
+ *
+ * One chunk of it, blocks [lo, lo + cnt) already in HBM at d_blocks (work enqueued on ctx->stream, ctx->mu held).
+ * d_pre_status (may be NULL): a status per block from before the encoders (the block build); a block that failed
+ * there keeps it, asks alloc for no page and writes nothing.  d_blk / h_blk: cnt * cap_pages block numbers of
+ * device / pinned staging for the page rows.
  */
+static int
+flush_chunk(cryogpu_ctx *ctx, size_t lo, size_t cnt, int method, int level_or_accel, const uint8_t *d_blocks,
+            uint64_t stride, uint32_t block_size, const int32_t *d_pre_status, uint32_t *d_blk, uint32_t *h_blk,
+            const uint32_t *first_blkno, cryogpu_alloc_page_fn alloc, cryogpu_page_ptr_fn page_ptr, void *arg,
+            uint32_t created_xid, uint32_t *npages, uint32_t *comp_size, int32_t *status, uint64_t &h2d, uint64_t &d2h)
+{
+    const uint64_t bound = cryogpu_compress_bound(method, block_size), cstride = (bound + 15) & ~(uint64_t) 15;
+    const uint32_t cap_pages = pg_pages_needed(bound);
+    const size_t   pstride = (size_t) cap_pages * PG_PAGE, meta = (cnt * 12 + 255) & ~(size_t) 255;
+    int            rc;
+
+    if ((rc = host_reserve(ctx->h_out[0], cnt * pstride + meta)) != CRYOGPU_OK ||
+        (rc = dev_reserve(ctx->d_out[0], cnt * pstride + meta)) != CRYOGPU_OK ||
+        (rc = dev_reserve(ctx->pgw, cnt * cstride + meta)) != CRYOGPU_OK)
+        return rc;
+    uint8_t  *ho = (uint8_t *) ctx->h_out[0].p, *dout = (uint8_t *) ctx->d_out[0].p;
+    uint8_t  *comp = (uint8_t *) ctx->pgw.p, *dm = dout + cnt * pstride;
+    uint32_t *d_np = (uint32_t *) dm, *d_cs = (uint32_t *) (dm + cnt * 4);
+    int32_t  *d_st = (int32_t *) (dm + cnt * 8), *d_cst = (int32_t *) (comp + cnt * cstride);
+    const uint8_t *hm = ho + cnt * pstride;
+
+    CU(cudaStreamWaitEvent(ctx->stream, ctx->busy, 0));
+    rc = compress_device_locked(ctx, ctx->stream, cnt, method, level_or_accel, d_blocks, stride, block_size, comp, cstride,
+                                (uint32_t) cstride, d_cs, d_cst);
+    if (rc != CRYOGPU_OK)
+        return rc;
+    /* a failed build overrides what the encoders made of the unwritten block: its status, compressed size 0 */
+    if (d_pre_status)
+    {
+        k_pages_status<<<(unsigned) ((cnt + 255) / 256), 256, 0, ctx->stream>>>(d_pre_status, nullptr, d_cst, d_cs, nullptr,
+                                                                               (uint32_t) cnt);
+        CU(cudaGetLastError());
+    }
+    CU(cudaMemcpyAsync(ho + cnt * pstride + cnt * 4, d_cs, cnt * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    CU(cudaStreamSynchronize(ctx->stream));
+    d2h += cnt * 4;
+    /* the block numbers, in the order cryo_preserve takes them: block by block, page by page */
+    const uint32_t *h_cs = (const uint32_t *) (hm + cnt * 4);
+
+    for (size_t i = 0; i < cnt; i++)
+    {
+        const uint32_t np = pg_pages_needed(h_cs[i]);
+
+        h_blk[i * cap_pages] = first_blkno[lo + i];
+        for (uint32_t k = 1; k < cap_pages; k++)
+            h_blk[i * cap_pages + k] = k < np ? alloc(arg) : PG_INVALID;
+    }
+    CU(cudaMemcpyAsync(d_blk, h_blk, cnt * cap_pages * 4, cudaMemcpyHostToDevice, ctx->stream));
+    h2d += cnt * cap_pages * 4;
+    k_pages_split<<<(unsigned) cnt, 256, 0, ctx->stream>>>(comp, cstride, d_cs, d_cst, (uint32_t) method, created_xid, d_blk,
+                                                          cap_pages, dout, pstride, d_np, d_st);
+    CU(cudaGetLastError());
+    CU(cudaEventRecord(ctx->busy, ctx->stream));
+    CU(cudaMemcpyAsync(ho + cnt * pstride, dm, meta, cudaMemcpyDeviceToHost, ctx->stream));
+    for (size_t i = 0; i < cnt; i++)
+    {
+        const uint32_t np = pg_pages_needed(h_cs[i]);
+
+        CU(cudaMemcpyAsync(ho + i * pstride, dout + i * pstride, (size_t) np * PG_PAGE, cudaMemcpyDeviceToHost, ctx->stream));
+        d2h += (size_t) np * PG_PAGE;
+    }
+    CU(cudaStreamSynchronize(ctx->stream));
+    d2h += meta;
+    memcpy(npages + lo, hm, cnt * 4);
+    memcpy(comp_size + lo, hm + cnt * 4, cnt * 4);
+    memcpy(status + lo, hm + cnt * 8, cnt * 4);
+    for (size_t i = 0; i < cnt; i++)
+        if (status[lo + i] == CRYOGPU_ST_OK)
+            for (uint32_t k = 0; k < npages[lo + i]; k++)
+            {
+                void *p = page_ptr(arg, h_blk[i * cap_pages + k]);
+
+                if (!p)
+                    return fail(CRYOGPU_E_ARG, "page_ptr returned NULL for block %u", h_blk[i * cap_pages + k]);
+                memcpy(p, ho + i * pstride + (size_t) k * PG_PAGE, PG_PAGE);
+            }
+    return CRYOGPU_OK;
+}
+
 extern "C" int
 cryogpu_compress_pages_alloc_host(cryogpu_ctx *ctx, size_t n, int method, int level_or_accel, const void *const *src,
                                   uint32_t block_size, const uint32_t *first_blkno, cryogpu_alloc_page_fn alloc,
@@ -2254,9 +2350,7 @@ cryogpu_compress_pages_alloc_host(cryogpu_ctx *ctx, size_t n, int method, int le
     if (block_size == 0 || block_size > (1u << 27))
         return fail(CRYOGPU_E_ARG, "block_size out of range");
     const uint64_t stride = ((uint64_t) block_size + 15) & ~(uint64_t) 15;
-    const uint64_t bound = cryogpu_compress_bound(method, block_size), cstride = (bound + 15) & ~(uint64_t) 15;
-    const uint32_t cap_pages = pg_pages_needed(bound);
-    const size_t   pstride = (size_t) cap_pages * PG_PAGE;
+    const uint32_t cap_pages = pg_pages_needed(cryogpu_compress_bound(method, block_size));
     uint64_t       h2d = 0, d2h = 0;
     std::lock_guard<std::recursive_mutex> hold(ctx->mu);
 
@@ -2264,24 +2358,15 @@ cryogpu_compress_pages_alloc_host(cryogpu_ctx *ctx, size_t n, int method, int le
     for (size_t lo = 0; lo < n; lo += PG_HOST_CHUNK)
     {
         const size_t cnt = std::min<size_t>(PG_HOST_CHUNK, n - lo);
-        const size_t blk_bytes = (cnt * cap_pages * 4 + 255) & ~(size_t) 255, meta = (cnt * 12 + 255) & ~(size_t) 255;
+        const size_t blk_bytes = (cnt * cap_pages * 4 + 255) & ~(size_t) 255;
         int          rc;
 
         if ((rc = host_reserve(ctx->h_in[0], cnt * stride + blk_bytes)) != CRYOGPU_OK ||
-            (rc = dev_reserve(ctx->d_in[0], cnt * stride + blk_bytes)) != CRYOGPU_OK ||
-            (rc = host_reserve(ctx->h_out[0], cnt * pstride + meta)) != CRYOGPU_OK ||
-            (rc = dev_reserve(ctx->d_out[0], cnt * pstride + meta)) != CRYOGPU_OK ||
-            (rc = dev_reserve(ctx->pgw, cnt * cstride + meta)) != CRYOGPU_OK)
+            (rc = dev_reserve(ctx->d_in[0], cnt * stride + blk_bytes)) != CRYOGPU_OK)
             return rc;
-        uint8_t  *hi = (uint8_t *) ctx->h_in[0].p, *di = (uint8_t *) ctx->d_in[0].p;
-        uint8_t  *ho = (uint8_t *) ctx->h_out[0].p, *dout = (uint8_t *) ctx->d_out[0].p;
-        uint8_t  *comp = (uint8_t *) ctx->pgw.p, *dm = dout + cnt * pstride;
-        uint32_t *d_np = (uint32_t *) dm, *d_cs = (uint32_t *) (dm + cnt * 4);
-        int32_t  *d_st = (int32_t *) (dm + cnt * 8), *d_cst = (int32_t *) (comp + cnt * cstride);
-        uint32_t *h_blk = (uint32_t *) (hi + cnt * stride);
-        const uint8_t *hm = ho + cnt * pstride;
+        uint8_t *hi = (uint8_t *) ctx->h_in[0].p, *di = (uint8_t *) ctx->d_in[0].p;
 
-        if (is_pinned(src[lo]))                         /* the batched writer's blocks are */
+        if (is_pinned(src[lo]))                         /* callers that hold pinned block images */
             for (size_t i = 0; i < cnt; i++)
                 CU(cudaMemcpyAsync(di + i * stride, src[lo + i], block_size, cudaMemcpyHostToDevice, ctx->stream));
         else
@@ -2290,55 +2375,169 @@ cryogpu_compress_pages_alloc_host(cryogpu_ctx *ctx, size_t n, int method, int le
             CU(cudaMemcpyAsync(di, hi, cnt * stride, cudaMemcpyHostToDevice, ctx->stream));
         }
         h2d += cnt * stride;
-        CU(cudaStreamWaitEvent(ctx->stream, ctx->busy, 0));
-        rc = compress_device_locked(ctx, ctx->stream, cnt, method, level_or_accel, di, stride, block_size, comp, cstride,
-                                    (uint32_t) cstride, d_cs, d_cst);
+        rc = flush_chunk(ctx, lo, cnt, method, level_or_accel, di, stride, block_size, nullptr, (uint32_t *) (di + cnt * stride),
+                         (uint32_t *) (hi + cnt * stride), first_blkno, alloc, page_ptr, arg, created_xid, npages, comp_size,
+                         status, h2d, d2h);
         if (rc != CRYOGPU_OK)
             return rc;
-        CU(cudaMemcpyAsync(ho + cnt * pstride + cnt * 4, d_cs, cnt * 4, cudaMemcpyDeviceToHost, ctx->stream));
-        CU(cudaStreamSynchronize(ctx->stream));
-        d2h += cnt * 4;
-        /* the block numbers, in the order cryo_preserve takes them: block by block, page by page */
-        const uint32_t *h_cs = (const uint32_t *) (hm + cnt * 4);
+    }
+    ctx->last_h2d = h2d;
+    ctx->last_d2h = d2h;
+    return CRYOGPU_OK;
+}
 
-        for (size_t i = 0; i < cnt; i++)
+/* ------------------------------------------------ cryo blocks from packed tuples */
+
+/* entry (off, len) of a batch whose data is data_size bytes: can its tuple go into a block of block_size bytes? */
+static bool
+entry_in_data(uint64_t off, uint32_t len, uint64_t data_size, uint32_t block_size)
+{
+    return off != UINT64_MAX && len <= block_size && off <= data_size && len <= data_size - off;
+}
+
+extern "C" int
+cryogpu_build_blocks_device(cryogpu_ctx *ctx, size_t n, const uint8_t *d_data, uint64_t data_size, const uint64_t *d_tup_off,
+                            const uint32_t *d_tup_len, const uint64_t *d_block_first, uint32_t block_size, uint8_t *d_dst,
+                            uint64_t dst_stride, int32_t *d_status, void *stream)
+{
+    if (!ctx)
+        return fail(CRYOGPU_E_ARG, "ctx is NULL");
+    if (block_size < 16 || block_size > (1u << 27) || (block_size & 7) || n > 0x7fffffffu)
+        return fail(CRYOGPU_E_ARG, "block_size must be a multiple of 8 in [16, 128 MiB]");
+    if (n == 0)
+        return CRYOGPU_OK;
+    if ((data_size && !d_data) || !d_tup_off || !d_tup_len || !d_block_first || !d_dst || !d_status)
+        return fail(CRYOGPU_E_ARG, "NULL device pointer");
+    if (((uintptr_t) d_dst & 15) || (dst_stride & 15) || dst_stride < block_size || ((uintptr_t) d_tup_off & 7) ||
+        ((uintptr_t) d_block_first & 7) || ((uintptr_t) d_tup_len & 3))
+        return fail(CRYOGPU_E_ARG, "d_dst, dst_stride multiples of 16, stride >= block_size; tup_off, block_first 8-byte aligned");
+    cudaStream_t st = stream ? (cudaStream_t) stream : ctx->stream;
+
+    CU(cudaSetDevice(ctx->device));
+    std::lock_guard<std::recursive_mutex> g(ctx->mu);
+
+    CU(cudaStreamWaitEvent(st, ctx->busy, 0));
+    k_block_build<<<(unsigned) n, BLK_THREADS, BLK_SMEM, st>>>(d_data, 0, data_size, (const tup_u64 *) d_tup_off, d_tup_len,
+                                                              (const tup_u64 *) d_block_first, block_size, d_dst, dst_stride,
+                                                              d_status);
+    CU(cudaGetLastError());
+    CU(cudaEventRecord(ctx->busy, st));
+    return CRYOGPU_OK;
+}
+
+/*
+ * The COPY flush from packed tuples.  Per chunk the bus carries the chunk's entries, its block_first row and the byte
+ * span of data its well-formed entries cover (for a writer that appends in order: exactly the chunk's tuples, about
+ * 22 KB per block of narrow rows against the 1 MiB image); the blocks are built in HBM and go through flush_chunk.
+ */
+extern "C" int
+cryogpu_compress_tuples_pages_alloc_host(cryogpu_ctx *ctx, size_t n, int method, int level_or_accel, const void *data,
+                                         uint64_t data_size, const uint64_t *tup_off, const uint32_t *tup_len,
+                                         const uint64_t *block_first, uint32_t block_size, const uint32_t *first_blkno,
+                                         cryogpu_alloc_page_fn alloc, cryogpu_page_ptr_fn page_ptr, void *arg,
+                                         uint32_t created_xid, uint32_t *npages, uint32_t *comp_size, int32_t *status)
+{
+    if (!ctx)
+        return fail(CRYOGPU_E_ARG, "ctx is NULL");
+    if (method != CRYOGPU_LZ4 && method != CRYOGPU_ZSTD)
+        return fail(CRYOGPU_E_METHOD, "unknown compression method %d", method);
+    if (block_size < 16 || block_size > (1u << 27) || (block_size & 7))
+        return fail(CRYOGPU_E_ARG, "block_size must be a multiple of 8 in [16, 128 MiB]");
+    if (n == 0)
+        return CRYOGPU_OK;
+    if (!block_first || !first_blkno || !alloc || !page_ptr || !npages || !comp_size || !status)
+        return fail(CRYOGPU_E_ARG, "NULL argument");
+    for (size_t i = 0; i < n; i++)
+        if (block_first[i + 1] < block_first[i])
+            return fail(CRYOGPU_E_ARG, "block_first must not decrease");
+    if (block_first[n] > block_first[0] && (!tup_off || !tup_len || (data_size && !data)))
+        return fail(CRYOGPU_E_ARG, "NULL argument");
+    const uint64_t stride = ((uint64_t) block_size + 15) & ~(uint64_t) 15;
+    const uint32_t cap_pages = pg_pages_needed(cryogpu_compress_bound(method, block_size));
+    uint64_t       h2d = 0, d2h = 0;
+    std::lock_guard<std::recursive_mutex> hold(ctx->mu);
+
+    CU(cudaSetDevice(ctx->device));
+    const bool data_pinned = data && is_pinned(data), ent_pinned = tup_off && is_pinned(tup_off) && is_pinned(tup_len);
+
+    for (size_t lo = 0; lo < n; lo += PG_HOST_CHUNK)
+    {
+        const size_t   cnt = std::min<size_t>(PG_HOST_CHUNK, n - lo);
+        const uint64_t e0 = block_first[lo], ne = block_first[lo + cnt] - e0;
+        uint64_t       b0 = UINT64_MAX, b1 = 0;
+
+        /* the bytes the chunk's well-formed entries cover, from a 16-byte boundary (the kernel rejects the others) */
+        for (uint64_t e = e0; e < e0 + ne; e++)
+            if (tup_len[e] && entry_in_data(tup_off[e], tup_len[e], data_size, block_size))
+            {
+                b0 = std::min(b0, tup_off[e]);
+                b1 = std::max(b1, tup_off[e] + tup_len[e]);
+            }
+        b0 = b0 == UINT64_MAX ? 0 : b0 & ~(uint64_t) 15;
+        b1 = std::max(b0, b1);
+        /* device: blocks | page rows | block_first (cnt + 1) | tup_off | tup_len | status | span (+ 16: the copies read
+         * whole aligned words); pinned staging: page rows | block_first | tup_off, tup_len, span if the caller's are not */
+        const size_t blk_bytes = tp_al(cnt * cap_pages * 4), bf_bytes = tp_al((cnt + 1) * 8), to_bytes = tp_al(ne * 8),
+                     tl_bytes = tp_al(ne * 4), st_bytes = tp_al(cnt * 4), span = b1 - b0, sp_bytes = tp_al(span + 16);
+        const size_t d_total = cnt * stride + blk_bytes + bf_bytes + to_bytes + tl_bytes + st_bytes + sp_bytes;
+        const size_t h_total = blk_bytes + bf_bytes + (ent_pinned ? 0 : to_bytes + tl_bytes) + (data_pinned ? 0 : sp_bytes);
+        int          rc;
+
+        if ((rc = host_reserve(ctx->h_in[0], h_total)) != CRYOGPU_OK || (rc = dev_reserve(ctx->d_in[0], d_total)) != CRYOGPU_OK)
+            return rc;
+        uint8_t  *hi = (uint8_t *) ctx->h_in[0].p, *di = (uint8_t *) ctx->d_in[0].p;
+        uint32_t *d_blk = (uint32_t *) (di + cnt * stride);
+        uint64_t *d_bf = (uint64_t *) ((uint8_t *) d_blk + blk_bytes), *d_to = (uint64_t *) ((uint8_t *) d_bf + bf_bytes);
+        uint32_t *d_tl = (uint32_t *) ((uint8_t *) d_to + to_bytes);
+        int32_t  *d_bst = (int32_t *) ((uint8_t *) d_tl + tl_bytes);
+        uint8_t  *d_span = (uint8_t *) d_bst + st_bytes;
+        uint64_t *h_bf = (uint64_t *) (hi + blk_bytes);
+        uint8_t  *h_rest = (uint8_t *) h_bf + bf_bytes;
+        const uint64_t *src_to = tup_off + e0;
+        const uint32_t *src_tl = tup_len + e0;
+        const uint8_t  *src_span = (const uint8_t *) data + b0;
+
+        for (size_t i = 0; i <= cnt; i++)
+            h_bf[i] = block_first[lo + i] - e0;
+        if (!ent_pinned && ne)
         {
-            const uint32_t np = pg_pages_needed(h_cs[i]);
-
-            h_blk[i * cap_pages] = first_blkno[lo + i];
-            for (uint32_t k = 1; k < cap_pages; k++)
-                h_blk[i * cap_pages + k] = k < np ? alloc(arg) : PG_INVALID;
+            memcpy(h_rest, src_to, ne * 8);
+            memcpy(h_rest + to_bytes, src_tl, ne * 4);
+            src_to = (const uint64_t *) h_rest;
+            src_tl = (const uint32_t *) (h_rest + to_bytes);
+            h_rest += to_bytes + tl_bytes;
         }
-        CU(cudaMemcpyAsync(di + cnt * stride, h_blk, cnt * cap_pages * 4, cudaMemcpyHostToDevice, ctx->stream));
-        h2d += cnt * cap_pages * 4;
-        k_pages_split<<<(unsigned) cnt, 256, 0, ctx->stream>>>(comp, cstride, d_cs, d_cst, (uint32_t) method, created_xid,
-                                                              (uint32_t *) (di + cnt * stride), cap_pages, dout, pstride, d_np,
-                                                              d_st);
+        if (!data_pinned && span)
+        {
+            host_pool(ctx)->run((span + (1u << 20) - 1) >> 20, [&](size_t part) {
+                const size_t at = part << 20;
+
+                memcpy(h_rest + at, src_span + at, std::min<size_t>(1u << 20, span - at));
+            });
+            src_span = h_rest;
+        }
+        CU(cudaMemcpyAsync(d_bf, h_bf, (cnt + 1) * 8, cudaMemcpyHostToDevice, ctx->stream));
+        h2d += (cnt + 1) * 8;
+        if (ne)
+        {
+            CU(cudaMemcpyAsync(d_to, src_to, ne * 8, cudaMemcpyHostToDevice, ctx->stream));
+            CU(cudaMemcpyAsync(d_tl, src_tl, ne * 4, cudaMemcpyHostToDevice, ctx->stream));
+            h2d += ne * 12;
+        }
+        if (span)
+        {
+            CU(cudaMemcpyAsync(d_span, src_span, span, cudaMemcpyHostToDevice, ctx->stream));
+            h2d += span;
+        }
+        CU(cudaStreamWaitEvent(ctx->stream, ctx->busy, 0));
+        k_block_build<<<(unsigned) cnt, BLK_THREADS, BLK_SMEM, ctx->stream>>>(d_span, b0, data_size, (const tup_u64 *) d_to, d_tl,
+                                                                             (const tup_u64 *) d_bf, block_size, di, stride,
+                                                                             d_bst);
         CU(cudaGetLastError());
-        CU(cudaEventRecord(ctx->busy, ctx->stream));
-        CU(cudaMemcpyAsync(ho + cnt * pstride, dm, meta, cudaMemcpyDeviceToHost, ctx->stream));
-        for (size_t i = 0; i < cnt; i++)
-        {
-            const uint32_t np = pg_pages_needed(h_cs[i]);
-
-            CU(cudaMemcpyAsync(ho + i * pstride, dout + i * pstride, (size_t) np * PG_PAGE, cudaMemcpyDeviceToHost, ctx->stream));
-            d2h += (size_t) np * PG_PAGE;
-        }
-        CU(cudaStreamSynchronize(ctx->stream));
-        d2h += meta;
-        memcpy(npages + lo, hm, cnt * 4);
-        memcpy(comp_size + lo, hm + cnt * 4, cnt * 4);
-        memcpy(status + lo, hm + cnt * 8, cnt * 4);
-        for (size_t i = 0; i < cnt; i++)
-            if (status[lo + i] == CRYOGPU_ST_OK)
-                for (uint32_t k = 0; k < npages[lo + i]; k++)
-                {
-                    void *p = page_ptr(arg, h_blk[i * cap_pages + k]);
-
-                    if (!p)
-                        return fail(CRYOGPU_E_ARG, "page_ptr returned NULL for block %u", h_blk[i * cap_pages + k]);
-                    memcpy(p, ho + i * pstride + (size_t) k * PG_PAGE, PG_PAGE);
-                }
+        rc = flush_chunk(ctx, lo, cnt, method, level_or_accel, di, stride, block_size, d_bst, d_blk, (uint32_t *) hi, first_blkno,
+                         alloc, page_ptr, arg, created_xid, npages, comp_size, status, h2d, d2h);
+        if (rc != CRYOGPU_OK)
+            return rc;
     }
     ctx->last_h2d = h2d;
     ctx->last_d2h = d2h;

@@ -581,44 +581,35 @@ struct CryoBatchWriter
     const CryoRelOps *ops;
     int         method, level, batch;
     uint32_t    xid;
-    char      **data;           /* batch + 1 blocks, pinned; [nfull] is the one being filled */
+    /* the tuples of the queued blocks and the current one, appended MAXALIGNed, and their entries; pinned, sized at
+     * create for batch + 1 blocks (a block holds under CRYO_BATCH_BLCKSZ bytes of tuples and at most 290 items) */
+    uint8_t    *tup;
+    uint64_t   *tup_off, *block_first;  /* block_first[k]: the first entry of queued block k */
+    uint32_t   *tup_len;
+    uint64_t    nent, nbytes;
+    uint32_t    lower, upper;           /* storage.c's two counters of the current block */
     uint32_t   *target_block;   /* reserved first page of each (pg_cryogen.c:588-601) */
     int         nfull;
     int         started;        /* the current block has a reserved page */
     uint64_t    calls, blocks, pages;
-    double      flush_seconds;  /* spent in the device calls (compress + split + copies), for benchmarks */
+    double      flush_seconds;  /* spent in the device calls (build + compress + split + copies), for benchmarks */
 };
 
-/* cryo_init_page, storage.c:15-21 */
-static void
-init_block(char *d)
-{
-    uint32_t lower = 8, upper = CRYO_BATCH_BLCKSZ;
-
-    memset(d, 0, CRYO_BATCH_BLCKSZ);
-    memcpy(d, &lower, 4);
-    memcpy(d + 4, &upper, 4);
-}
-
-/* cryo_storage_insert, storage.c:26-50.  sizeof(ItemId) there is the size of a POINTER (ItemId is ItemIdData *):
- * 8 bytes, which happens to be sizeof(CryoItemId); MaxHeapTuplesPerPage = 291 for 8 KiB pages. */
+/* cryo_storage_insert, storage.c:26-50, on the current block's counters: the device builds the block image from the
+ * entries at flush time.  sizeof(ItemId) there is the size of a POINTER (ItemId is ItemIdData *): 8 bytes, which
+ * happens to be sizeof(CryoItemId); MaxHeapTuplesPerPage = 291 for 8 KiB pages. */
 static int
-storage_insert(char *d, const void *tuple, uint32_t len)
+storage_insert(CryoBatchWriter *w, const void *tuple, uint32_t len)
 {
-    uint32_t lower, upper;
-
-    memcpy(&lower, d, 4);
-    memcpy(&upper, d + 4, 4);
-    if (len + 8u > upper - lower || (lower - 8u) / 8u + 1u >= 291u)
+    if (len + 8u > w->upper - w->lower || (w->lower - 8u) / 8u + 1u >= 291u)
         return -1;
-    upper -= (len + 7u) & ~7u;                  /* MAXALIGN */
-    memcpy(d + upper, tuple, len);
-    memcpy(d + lower, &upper, 4);
-    memcpy(d + lower + 4, &len, 4);
-    lower += 8;                                 /* d->lower += sizeof(ItemId), storage.c:47 */
-    memcpy(d, &lower, 4);
-    memcpy(d + 4, &upper, 4);
-    return (int) ((lower - 8u) / 8u);
+    w->upper -= (len + 7u) & ~7u;               /* MAXALIGN */
+    memcpy(w->tup + w->nbytes, tuple, len);
+    w->tup_off[w->nent] = w->nbytes;
+    w->tup_len[w->nent++] = len;
+    w->nbytes += (len + 7u) & ~7u;
+    w->lower += 8;                              /* d->lower += sizeof(ItemId), storage.c:47 */
+    return (int) ((w->lower - 8u) / 8u);
 }
 
 CryoBatchWriter *
@@ -629,28 +620,34 @@ cryo_batch_writer_create(cryogpu_ctx *gpu, const CryoRelOps *ops, int method, in
 
     if (!w || batch_blocks < 1)
         return NULL;
+    const size_t blocks = (size_t) batch_blocks + 1;
+
     w->gpu = gpu;
     w->ops = ops;
     w->method = method;
     w->level = level_or_accel;
     w->batch = batch_blocks;
     w->xid = xid;
-    w->data = calloc((size_t) batch_blocks + 1, sizeof(char *));
-    w->target_block = calloc((size_t) batch_blocks + 1, sizeof(uint32_t));
-    for (int i = 0; w->data && i <= batch_blocks; i++)
-        if (!(w->data[i] = cryogpu_host_alloc(CRYO_BATCH_BLCKSZ)))
-        {
-            cryo_batch_writer_destroy(w);
-            return NULL;
-        }
+    w->target_block = calloc(blocks, sizeof(uint32_t));
+    w->block_first = calloc(blocks + 1, sizeof(uint64_t));
+    w->tup = cryogpu_host_alloc(blocks * CRYO_BATCH_BLCKSZ);
+    w->tup_off = cryogpu_host_alloc(blocks * 290 * sizeof(uint64_t));
+    w->tup_len = cryogpu_host_alloc(blocks * 290 * sizeof(uint32_t));
+    if (!w->target_block || !w->block_first || !w->tup || !w->tup_off || !w->tup_len)
+    {
+        cryo_batch_writer_destroy(w);
+        return NULL;
+    }
     return w;
 }
 
-/* init_modify_state, pg_cryogen.c:603-617: a fresh block and its reserved first page */
+/* init_modify_state, pg_cryogen.c:603-617: a fresh block (cryo_init_page's counters) and its reserved first page */
 static void
 start_block(CryoBatchWriter *w)
 {
-    init_block(w->data[w->nfull]);
+    w->lower = 8;
+    w->upper = CRYO_BATCH_BLCKSZ;
+    w->block_first[w->nfull] = w->nent;
     w->target_block[w->nfull] = w->ops->extend(w->ops->rel);
     w->started = 1;
 }
@@ -658,6 +655,7 @@ start_block(CryoBatchWriter *w)
 static uint32_t alloc_cb(void *arg) { CryoBatchWriter *w = arg; return w->ops->extend(w->ops->rel); }
 static void *ptr_cb(void *arg, uint32_t blkno) { CryoBatchWriter *w = arg; return w->ops->read_page(w->ops->rel, blkno); }
 
+/* the n queued blocks, which hold every entry so far; the packed buffer starts over */
 static int
 flush_blocks(CryoBatchWriter *w, int n)
 {
@@ -667,13 +665,15 @@ flush_blocks(CryoBatchWriter *w, int n)
     int32_t  *st = malloc(sizeof(int32_t) * (size_t) n);
     int       rc = CRYOGPU_E_NOMEM;
 
+    w->block_first[n] = w->nent;
     if (np && st)
     {
         struct timespec t0, t1;
 
         clock_gettime(CLOCK_MONOTONIC, &t0);
-        rc = cryogpu_compress_pages_alloc_host(w->gpu, (size_t) n, w->method, w->level, (const void *const *) w->data,
-                                               CRYO_BATCH_BLCKSZ, w->target_block, alloc_cb, ptr_cb, w, w->xid, np, np + n, st);
+        rc = cryogpu_compress_tuples_pages_alloc_host(w->gpu, (size_t) n, w->method, w->level, w->tup, w->nbytes, w->tup_off,
+                                                      w->tup_len, w->block_first, CRYO_BATCH_BLCKSZ, w->target_block,
+                                                      alloc_cb, ptr_cb, w, w->xid, np, np + n, st);
         clock_gettime(CLOCK_MONOTONIC, &t1);
         w->flush_seconds += (double) (t1.tv_sec - t0.tv_sec) + 1e-9 * (double) (t1.tv_nsec - t0.tv_nsec);
         w->calls++;
@@ -685,6 +685,8 @@ flush_blocks(CryoBatchWriter *w, int n)
         }
         w->blocks += (uint64_t) n;
     }
+    w->nent = 0;
+    w->nbytes = 0;
     free(np);
     free(st);
     return rc;
@@ -697,7 +699,7 @@ cryo_batch_insert(CryoBatchWriter *w, const void *tuple, uint32_t len, uint32_t 
 
     if (!w->started)
         start_block(w);
-    if ((pos = storage_insert(w->data[w->nfull], tuple, len)) < 0)
+    if ((pos = storage_insert(w, tuple, len)) < 0)
     {
         /* pg_cryogen.c:634-647: the block is full.  The reference compresses and writes it now; here it waits
          * for its batch. */
@@ -712,7 +714,7 @@ cryo_batch_insert(CryoBatchWriter *w, const void *tuple, uint32_t len, uint32_t 
                 return rc;
         }
         start_block(w);
-        if ((pos = storage_insert(w->data[w->nfull], tuple, len)) < 0)
+        if ((pos = storage_insert(w, tuple, len)) < 0)
             return -1;                          /* "tuple is too large to fit the cryo block" */
     }
     *tid_block = w->target_block[w->nfull];
@@ -768,9 +770,10 @@ cryo_batch_writer_destroy(CryoBatchWriter *w)
 {
     if (!w)
         return;
-    for (int i = 0; w->data && i <= w->batch; i++)
-        cryogpu_host_free(w->data[i]);
-    free(w->data);
+    cryogpu_host_free(w->tup);
+    cryogpu_host_free(w->tup_off);
+    cryogpu_host_free(w->tup_len);
+    free(w->block_first);
     free(w->target_block);
     free(w);
 }

@@ -15,9 +15,11 @@
  *               the next block numbers.
  *   write side  a modify state that keeps several full 1 MiB blocks (the reference flushes at the
  *               first full one, pg_cryogen.c:634-640) and hands them to ONE
- *               cryogpu_compress_pages_alloc_host call; the first page of every block is reserved when
+ *               cryogpu_compress_tuples_pages_alloc_host call; the first page of every block is reserved when
  *               the block is started, as cryo_reserve_blockno does (pg_cryogen.c:588-601), because
- *               the item pointers of its tuples carry that number.
+ *               the item pointers of its tuples carry that number.  The blocks are kept as their tuples,
+ *               packed, with storage_insert's two counters per block deciding where one ends: the device
+ *               builds the block images, so only the tuple bytes cross the bus.
  *
  * PostgreSQL's buffer manager is reached through CryoRelOps, so the module builds and is tested
  * without a backend; INTEGRATION.md shows the ReadBuffer / BufferGetPage / P_NEW bindings.
