@@ -129,6 +129,8 @@ int cryogpu_decompress_device(cryogpu_ctx *ctx, size_t n,
  * d_src + i * src_stride (block_size bytes) and written to d_dst + i * dst_stride
  * (capacity dst_cap >= cryogpu_compress_bound).  level_or_accel is
  * lz4_acceleration (compression.c:72) or zstd_compression_level (compression.c:104).
+ * A block's stream depends only on its bytes, the method and level_or_accel: not on
+ * the other blocks of the batch, its place in it, or the bytes after it in its slot.
  */
 int cryogpu_compress_device(cryogpu_ctx *ctx, size_t n, int method, int level_or_accel,
                             const uint8_t *d_src, uint64_t src_stride, uint32_t block_size,

@@ -99,6 +99,20 @@ CRYO_DEV void lz4e_put_ext(uint8_t *p, uint32_t v, uint32_t lane)
 }
 
 /*
+ * table[h] = v for every lane with `on`, by the whole warp.  Where lanes share a slot the highest lane (the latest
+ * position, as liblz4's serial walk would leave it) writes alone: CUDA leaves unspecified which of several stores
+ * to one address lands, and a table that depended on it would make a block's stream depend on how the warps were
+ * scheduled, so on its neighbours in the batch.
+ */
+CRYO_DEV void lz4e_insert(uint16_t *table, uint32_t h, uint16_t v, bool on, uint32_t lane)
+{
+    const uint32_t peers = __match_any_sync(CRYO_FULL, on ? h : ~0u);
+
+    if (on && lane == 31u - (uint32_t) __clz((int) peers))
+        table[h] = v;
+}
+
+/*
  * One warp compresses in[0, len) (one segment) into the scratch stream `body`.
  * Matches never start after len - 12 and never cover the last 5 bytes (the LZ4 end
  * of block rules, applied to every segment so that any of them may be the last).
@@ -147,8 +161,7 @@ CRYO_DEV void lz4e_segment(const uint8_t *in, uint32_t len, uint32_t hist, int a
             {
                 const uint32_t q = q0 + (32u * u + lane) * hstep;
 
-                if (q < H)
-                    table[(v[u] * 2654435761u) >> (32 - LZ4E_HASHLOG)] = (uint16_t) q;
+                lz4e_insert(table, (v[u] * 2654435761u) >> (32 - LZ4E_HASHLOG), (uint16_t) q, q < H, lane);
             }
         }
         __syncwarp();
@@ -212,8 +225,7 @@ CRYO_DEV void lz4e_segment(const uint8_t *in, uint32_t len, uint32_t hist, int a
                 m = 1;              /* forced: position 0 continues a match at offset cont_off */
             /* insert the probed positions up to and including the first hit; the ones behind
              * it will be probed again after the match and must still see older candidates */
-            if (valid && (m & ((1u << lane) - 1u)) == 0)
-                table[h] = (uint16_t) (pos + H);
+            lz4e_insert(table, h, (uint16_t) (pos + H), valid && (m & ((1u << lane) - 1u)) == 0, lane);
             __syncwarp();
             if (m == 0)
             {

@@ -533,8 +533,15 @@ CRYO_DEV uint32_t zse_find_matches(const uint8_t *in, uint32_t len, const ZsePar
             const bool     use_rep = mr != 0 && kr <= kh + 1;
             const int      k = use_rep ? kr : kh;
 
-            if (valid && (int) lane <= (k > 31 ? 31 : k))
-                table[h] = (uint16_t) pos;
+            {
+                /* one store per slot, the highest lane's (see lz4e_insert: the winner of stores to one address
+                 * is unspecified, and the stream must not depend on scheduling) */
+                const bool     ins = valid && (int) lane <= (k > 31 ? 31 : k);
+                const uint32_t peers = __match_any_sync(CRYO_FULL, ins ? h : ~0u);
+
+                if (ins && lane == 31u - (uint32_t) __clz((int) peers))
+                    table[h] = (uint16_t) pos;
+            }
             __syncwarp();
             if (k > 31)
             {
@@ -576,17 +583,23 @@ CRYO_DEV uint32_t zse_find_matches(const uint8_t *in, uint32_t len, const ZsePar
             }
             p = anchor = mpos + ml;
             missed = 0;
-            if (lane < 2)
             {
-                /* like libzstd: remember match start + 2 and match end - 2 */
+                /* like libzstd: remember match start + 2 and then match end - 2 (the later one where both hash
+                 * to one slot) */
                 const uint32_t q = lane == 0 ? mpos + 2 : p - 2;
+                const bool     ins = lane < 2 && q <= plimit;
+                uint32_t       hq = ~0u;
 
-                if (q <= plimit)
+                if (ins)
                 {
                     uint32_t a = zse_ld4(in + q), b = zse_ld4(in + q + 4) & tailmask;
 
-                    table[((a * 2654435761u) ^ (b * 2246822519u)) >> (32 - ZSE_HASHLOG)] = (uint16_t) q;
+                    hq = ((a * 2654435761u) ^ (b * 2246822519u)) >> (32 - ZSE_HASHLOG);
                 }
+                const uint32_t h1 = __shfl_sync(CRYO_FULL, hq, 1);
+
+                if (ins && !(lane == 0 && h1 == hq))
+                    table[hq] = (uint16_t) q;
             }
             __syncwarp();
             /* immediate matches at the second repeat offset (no literals in between) */
