@@ -5,13 +5,26 @@ Each is (name, frame bytes as uint8 array, expected output bytes)."""
 import numpy as np
 
 
-def _frame(content_len, blocks):
-    """single-segment frame, 1-byte FCS (content_len < 256)"""
-    assert content_len < 256
-    return bytes([0x28, 0xB5, 0x2F, 0xFD, 0x20, content_len]) + b"".join(blocks)
+def _frame(content_len, blocks, fcs_bytes=1, window_log=None, checksum=None):
+    """A frame around the given blocks.  window_log None: single segment with a content size of fcs_bytes (1, 2, 4
+    or 8) bytes; otherwise a window descriptor of that log and a content size of fcs_bytes (0: none, 2, 4 or 8).
+    checksum: the 4 bytes written after the last block (sets the checksum flag)."""
+    if window_log is None:
+        flag = {1: 0, 2: 1, 4: 2, 8: 3}[fcs_bytes]
+        fhd, wd = 0x20 | (flag << 6), b""
+    else:
+        flag = {0: 0, 2: 1, 4: 2, 8: 3}[fcs_bytes]
+        fhd, wd = flag << 6, bytes([(window_log - 10) << 3])
+    if checksum is not None:
+        fhd |= 0x04
+    v = content_len - 256 if fcs_bytes == 2 else content_len
+    assert 0 <= v < 1 << (8 * fcs_bytes) or fcs_bytes == 0
+    return (bytes([0x28, 0xB5, 0x2F, 0xFD, fhd]) + wd + v.to_bytes(fcs_bytes, "little") + b"".join(blocks) +
+            (bytes(checksum) if checksum is not None else b""))
 
 
 def _block_header(last, btype, size):
+    """btype 0 Raw, 1 RLE, 2 Compressed; size: the bytes of a Raw or Compressed block, the count of an RLE one"""
     v = (1 if last else 0) | (btype << 1) | (size << 3)
     return bytes([v & 0xFF, (v >> 8) & 0xFF, (v >> 16) & 0xFF])
 
