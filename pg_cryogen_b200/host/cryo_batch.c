@@ -15,16 +15,25 @@
 #define OFF_FIRST    24
 #define OFF_NEXT     28
 #define OFF_XID      32
-#define OFF_NPAGES   44
+#define OFF_CSIZE    40
 
 static uint32_t rd32(const uint8_t *p) { uint32_t v; memcpy(&v, p, 4); return v; }
 static uint32_t rd16(const uint8_t *p) { uint16_t v; memcpy(&v, p, 2); return v; }
 
+/* cryo_pages_needed, pg_cryogen.c:692-704: the pages a chain of compressed_size bytes has */
+static uint32_t
+pages_needed(uint64_t size)
+{
+    return size <= CRYO_BATCH_PAGE - 48u ? 1u
+                                         : 1u + (uint32_t) ((size - (CRYO_BATCH_PAGE - 48u) + CRYO_BATCH_PAGE - 32u - 1u) / (CRYO_BATCH_PAGE - 32u));
+}
+
 /* ------------------------------------------------------------------ read side */
 
 /*
- * The pages of the chain that starts at blk, following `next` as cache.c:151-176 does: the device needs the pages, the
- * host finds them.  An empty or foreign first page still goes to the device alone: it names the error (cache.c:112-129).
+ * The pages of the chain that starts at blk, following `next` as cache.c:151-176 does, until compressed_size is covered
+ * (the reference never reads npages): the device needs the pages, the host finds them.  An empty or foreign first page
+ * still goes to the device alone: it names the error (cache.c:112-129).
  * Fills pages[] / pblk[] (CRYO_BATCH_MAXPAGES at most) and returns their number; *xid: created_xid of a first page.
  */
 static uint32_t
@@ -35,7 +44,7 @@ walk_chain(const CryoRelOps *ops, uint32_t blk, uint32_t relblocks, const void *
 
     if (pg && rd16(pg + OFF_PD_UPPER) != 0 && rd32(pg + OFF_FIRST) == blk)
     {
-        want = rd16(pg + OFF_NPAGES);
+        want = pages_needed(rd32(pg + OFF_CSIZE));
         *xid = rd32(pg + OFF_XID);
     }
     while (pg && k < CRYO_BATCH_MAXPAGES)
@@ -57,6 +66,8 @@ typedef struct
     uint32_t    blockno;        /* key (one relation per cache here; the reference keys by (relid, blockno)) */
     int         used;
     uint64_t    ts;             /* last use, for LRU (cache.c:37, :200-206) */
+    uint64_t    miss;           /* the call (its stamp) that took the slot for a miss ... */
+    int         req;            /* ... and that call's request that did */
     uint32_t    nblocks;        /* cache.c:39 */
     uint32_t    xid;            /* cache.c:40 */
     uint32_t    blocks[CRYO_BATCH_MAXPAGES];
@@ -168,7 +179,8 @@ cryo_batch_read_data(CryoBatchCache *c, const CryoRelOps *ops, const uint32_t *b
         {
             c->slot[e].ts = stamp;
             entries[i] = e;
-            c->hits++;
+            if (c->slot[e].miss != stamp)       /* a repeat of this call's miss is not a hit: see below */
+                c->hits++;
             continue;
         }
         e = take_slot(c, stamp);
@@ -182,6 +194,8 @@ cryo_batch_read_data(CryoBatchCache *c, const CryoRelOps *ops, const uint32_t *b
         s->used = 1;
         s->blockno = blocknos[i];
         s->ts = stamp;
+        s->miss = stamp;
+        s->req = i;
         s->nblocks = 0;
         entries[i] = e;
         miss[nmiss++] = i;
@@ -247,6 +261,17 @@ done:
             entries[miss[m]] = InvalidCacheEntry;
             errs[miss[m]] = CRYO_ERR_DECOMPRESSION_FAILED;
         }
+    /* a block named again after its miss in this call gets that miss's outcome: its error, and its entry or none */
+    for (int i = 0; i < n; i++)
+    {
+        const int e = entries[i];
+
+        if (e != InvalidCacheEntry && c->slot[e].miss == stamp && c->slot[e].req != i)
+        {
+            errs[i] = errs[c->slot[e].req];
+            entries[i] = entries[c->slot[e].req];
+        }
+    }
     free(miss);
     free(pages);
     free(pblk);
@@ -328,9 +353,9 @@ scan_fill(CryoBatchScan *s)
         /* follow the chain now, so that its later pages are not taken for starting pages */
         if (pg && rd16(pg + OFF_PD_UPPER) != 0 && rd32(pg + OFF_FIRST) == b)
         {
-            uint32_t want = rd16(pg + OFF_NPAGES), k = 1, nb = rd32(pg + OFF_NEXT);
+            uint32_t want = pages_needed(rd32(pg + OFF_CSIZE)), k = 1, nb = rd32(pg + OFF_NEXT);
 
-            while (k < want && nb != INVALID_BLOCK && nb < s->relblocks)
+            while (k < want && k < CRYO_BATCH_MAXPAGES && nb != INVALID_BLOCK && nb < s->relblocks)
             {
                 s->excluded[nb] = 1;
                 nb = rd32((const uint8_t *) s->ops->read_page(s->ops->rel, nb) + OFF_NEXT);

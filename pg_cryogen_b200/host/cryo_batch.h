@@ -63,7 +63,9 @@ typedef struct CryoBatchCache CryoBatchCache;
 CryoBatchCache *cryo_batch_cache_create(cryogpu_ctx *gpu, int nslots);
 void        cryo_batch_cache_destroy(CryoBatchCache *c);
 /* cache.c:244-297, for n blocks at once: the misses among blocknos[] are read, in one device call.
- * errs[i] is what cryo_read_data would have returned for blocknos[i]; entries[i] the slot (or InvalidCacheEntry). */
+ * errs[i] is what cryo_read_data would have returned for blocknos[i]; entries[i] the slot (or InvalidCacheEntry).
+ * A block number may repeat: a request for a block that an earlier request of the same call missed gets that
+ * miss's outcome (its error, and its entry or InvalidCacheEntry) and is not counted as a hit. */
 int         cryo_batch_read_data(CryoBatchCache *c, const CryoRelOps *ops, const uint32_t *blocknos, int n,
                                  CacheEntry *entries, CryoError *errs);
 /* cache.h:33-36 */
@@ -72,7 +74,7 @@ const uint32_t *cryo_batch_get_pg_blocks(CryoBatchCache *c, CacheEntry e);
 char       *cryo_batch_get_data(CryoBatchCache *c, CacheEntry e);
 uint32_t    cryo_batch_get_xid(CryoBatchCache *c, CacheEntry e);
 void        cryo_batch_cache_invalidate(CryoBatchCache *c);
-/* device calls made and blocks decompressed so far */
+/* device calls made, blocks decompressed and requests served from the cache so far */
 void        cryo_batch_cache_stats(const CryoBatchCache *c, uint64_t *calls, uint64_t *blocks, uint64_t *hits);
 
 /* sequential scan with read-ahead (cryo_getnextslot's block loop, pg_cryogen.c:253-291, over the iterator of
